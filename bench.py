@@ -4,7 +4,7 @@
 achieved HBM GB/s of the dominant gate pass against the measured B200 roofline and the
 CPU restatement of the reference path timed beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one circuit: product-state init (+H layer), the fused clique passes, the
@@ -416,6 +416,27 @@ def ranks_identical(dist, world, counts, p, delta):
     return all(g == got[0] for g in got)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays, limit=DUMP_BYTES):
+    """Write every array as dirname/<name>.npy in float64, at most `limit` bytes in all.  Integer arrays (sampled keys)
+    must be below 2^53 so that float64 holds them exactly.  An array too large for its share of the limit is replaced by
+    its entries at a fixed, seeded sample of positions, which go to <name>_index.npy."""
+    cap = limit // (8 * 2 * len(arrays))
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a).reshape(-1)
+        if a.dtype.kind in 'iu' and a.size and int(a.max()) >= 1 << 53:
+            raise ValueError('%s: integer values >= 2^53 have no exact float64 form' % name)
+        a = a.astype(np.float64)
+        if a.size > cap:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))
+            np.save(os.path.join(dirname, name + '_index.npy'), idx.astype(np.float64))
+            a = a[idx]
+        np.save(os.path.join(dirname, name + '.npy'), a)
+
+
 def workload_config(args, cliques, N):
     n = max(max(c) for c in cliques) + 1
     return {'workload': '%s: synthetic random-tree MRF, n=%d variables, k=%d pair cliques, N=%d total qubits, '
@@ -437,7 +458,14 @@ def main():
     ap.add_argument('--no-dense', action='store_true', help='skip the dense in-place gate-pass measurement')
     ap.add_argument('--dense-workload', default='q33')
     ap.add_argument('--dense-only', action='store_true', help='tuning aid: only the dense schedule, prints its dict')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last step of each timed arm returned as DIR/<name>.npy '
+                         '(float64), so that two builds can be compared output for output')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'b200' or args.dense_only or args.workload in ('fixtures', 'chain20')):
+        ap.error('--dump-outputs is implemented for the single-circuit workloads of --impl b200 only')
     if args.warmup < 3 and args.impl == 'b200':
         args.warmup = 3
 
@@ -579,6 +607,12 @@ def main():
     e2e_ms_mean, single_ms = (float(x) for x in e2e_t.cpu())
     clk = clocks.stop(c_lo, c_hi) if rank == 0 else None
     same = ranks_identical(dist if world > 1 else None, world, counts, p, delta)
+    if args.dump_outputs and rank == 0:
+        # device-timed arm: (sampled keys, post-selected pmf, success probability) of its last step; e2e arm: the last
+        # circuit of the list -- its pmf, success probability and counts (keys ascending)
+        ck = sorted((int(k, 2), v) for k, v in counts.items())
+        dump_outputs(args.dump_outputs, {'keys': out[0], 'pmf': out[1], 'delta': [out[2]], 'e2e_pmf': p, 'e2e_delta': [delta],
+                                         'e2e_count_keys': [k for k, _ in ck], 'e2e_counts': [v for _, v in ck]})
     last_timing = sim.last_timing() if hasattr(sim, 'last_timing') else None
     breakdown = getattr(sim, 'breakdown_ms', None)
     dense = None

@@ -8,6 +8,8 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <mutex>
+#include <set>
 #include <string>
 #include <vector>
 
@@ -1119,12 +1121,20 @@ static int launch_gather_inplace(qcm_handle h, const GatherArgs &a, const Gather
     auto kern = k_block_gather_inplace<R, V, M, 1, S>;
     const size_t smem = 256 + (size_t)S * (1 << M) * kGatherTileBytes + tab_bytes;
     if (smem > 227 * 1024) return fail(h, QCM_ERR_UNSUPPORTED, "gather ring needs %zu B of shared memory", smem);
-    // set once per kernel and size: changing a function's attributes while an instance of it is running (another rank's
-    // kernel on this GPU, already waiting for signals) would hold this launch back until that instance ends
-    static size_t attr_set = 0;
-    if (smem > attr_set) {
-        QCM_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_set = smem;
+    // set once per kernel and device, to the most any launch may ask for, before the first launch: changing a function's
+    // attributes while an instance of it is running (another rank's kernel on this GPU, already waiting for signals) would
+    // hold this launch back until that instance ends.  Ranks that share a process (threads, one handle each) get here
+    // concurrently, so the check and the set happen under one lock.
+    static std::mutex attr_mu;
+    static std::set<int> attr_set;
+    {
+        std::lock_guard<std::mutex> lock(attr_mu);
+        if (!attr_set.count(h->device)) {
+            int optin = 0;
+            QCM_CUDA(h, cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+            QCM_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
+            attr_set.insert(h->device);
+        }
     }
     const uint64_t tiles = ((1ull << (a.n_local - M)) / V) / kThreads;
     int K = env_int("QCM_GATHER_K", 16);

@@ -32,7 +32,7 @@ def test_library_exports_every_declared_symbol(native_built):
     assert lib.qcm_small_max_qubits(32) == 13 and lib.qcm_small_max_qubits(64) == 13
 
 
-def test_op_struct_layout_matches_header(native_built):
+def test_op_struct_layout_matches_header(native_built, tmp_path):
     """qcm_op as numpy sees it == as the C compiler lays it out."""
     src = r'''
     #include <stdio.h>
@@ -41,7 +41,7 @@ def test_op_struct_layout_matches_header(native_built):
     int main(void){ printf("%zu %zu %zu %zu %zu %zu", sizeof(qcm_op), offsetof(qcm_op, n_active_in),
         offsetof(qcm_op, ctrl), offsetof(qcm_op, table_off), sizeof(qcm_timing), offsetof(qcm_op, flags)); return 0; }
     '''
-    exe = '/tmp/qcm_layout_test'
+    exe = str(tmp_path / 'qcm_layout_test')
     subprocess.run(['gcc', '-x', 'c', '-', '-I', os.path.join(ROOT, 'include'), '-o', exe], input=src, text=True, check=True)
     vals = list(map(int, subprocess.run([exe], capture_output=True, text=True).stdout.split()))
     d = fusion.OP_DTYPE
