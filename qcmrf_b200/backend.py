@@ -29,6 +29,8 @@ from . import _native, fusion, ir, plancache
 __all__ = ['B200Simulator', 'Job', 'Result', 'Counts']
 
 _FUSION_MODES = ('off', 'clique', 'blocked')
+#: most sweep points one batched handle holds (the engine's limit: they are the grid's y dimension)
+SWEEP_MAX_POINTS = 65535
 
 
 class Counts(dict):
@@ -367,7 +369,8 @@ class B200Simulator:
     def _probs_from_handle(self, h, pr):
         pl = pr.plan
         n = pr.n_vars
-        ident = all(pl.layout[q] == q for q in range(n))
+        # variables that are never stored (|0> throughout) lie outside the state: the general marginal below pads them
+        ident = n <= pl.n_phys and all(pl.layout[q] == q for q in range(n))
         mask, value, _ = pr.ps
         if ident:
             return h.postselect(mask, value, n)
@@ -427,8 +430,10 @@ class B200Simulator:
         def pipeline(item):
             """item = (i, pr, prepare_ms) to enqueue, or None to drain."""
             nxt = None
-            if item is not None and pend[0] is not None and pend[0][1].plan.n_phys != item[1].plan.n_phys:
-                pipeline(None)                                # another state size replaces the handle: finish what is pending
+            if item is not None and pend[0] is not None and (pend[0][1].plan.n_phys != item[1].plan.n_phys or
+                                                             pend[0][1].n_vars != item[1].n_vars):
+                # another state size replaces the handle, another pmf size the result buffers: finish what is pending
+                pipeline(None)
             if item is not None:
                 i, pr, tp = item
                 te = time.perf_counter()
@@ -513,8 +518,8 @@ class B200Simulator:
         abytes = 8 if precision in ('single', 'c64', 32) else 16
         if (abytes << pl.n_phys) > self.sweep_state_bytes or len(pr.virtual) > 64:
             return None
-        if pr.ps is not None and not all(pl.layout[q] == q for q in range(pr.n_vars)):
-            return None                                       # the post-selected block must be the contiguous prefix
+        if pr.ps is not None and (pr.n_vars > pl.n_phys or not all(pl.layout[q] == q for q in range(pr.n_vars))):
+            return None                                       # the post-selected block must be the contiguous stored prefix
         rel = tuple((v['qubit'], tuple(v['ctrl'])) for v in pr.virtual)
         proj = (pr.proj[0].tobytes(), pr.proj[1].size) if pr.proj is not None else None
         return (pl.n_phys, pl.ops.tobytes(), pl.tables.size, pr.clbit_map.tobytes(), pr.ps, rel, proj, pr.prog.n_clbits)
@@ -693,7 +698,8 @@ class B200Simulator:
             sw = self._stack_sweep(prs)
         prs = sw.prs
         abytes = 8 if precision in ('single', 'c64', 32) else 16
-        cap = max(2, int(self.sweep_bytes // (abytes << sw.n_phys)))
+        # points per batched handle: sweep_bytes of state, and never more than the engine takes (qcm_create_batched)
+        cap = min(SWEEP_MAX_POINTS, max(2, int(self.sweep_bytes // (abytes << sw.n_phys))))
         entries = []
         n = len(prs)
         first = 0
@@ -768,7 +774,7 @@ class B200Simulator:
         precision = precision or self.precision
         h = self._handle(pl.n_phys, precision)
         n = pr.n_vars
-        if not (shots and not pr.virtual and pr.ps is not None and n is not None and n <= 30 and hasattr(h, 'mark')
+        if not (shots and not pr.virtual and pr.ps is not None and n is not None and n <= min(30, pl.n_phys) and hasattr(h, 'mark')
                 and all(pl.layout[q] == q for q in range(n))):
             out = self.execute(pr, shots, seed, stream, precision)
             return lambda: out

@@ -134,6 +134,16 @@ inline uint64_t btab(const qcm_sim_s *h) { return (uint64_t)h->tab_stride * real
 inline uint64_t btab64(const qcm_sim_s *h) { return (uint64_t)h->tab_stride * sizeof(double); }
 inline dim3 bgrid(const qcm_sim_s *h, uint64_t gx) { return dim3((unsigned)gx, (unsigned)h->batch, 1u); }
 inline uint64_t rank_bits(const qcm_sim_s *h) { return h->n_global ? (h->rank << h->n_local) : 0ull; }
+template <typename R> constexpr const char *real_name() { return sizeof(R) == 4 ? "float" : "double"; }
+// the op's kernel with its template arguments, for qcm_op_kernel_name
+inline void name_kernel(qcm_handle h, const char *fmt, ...) {
+    char nm[96];
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(nm, sizeof nm, fmt, ap);
+    va_end(ap);
+    h->cur_kernel = nm;
+}
 
 int grid_mult() {
     static int v = [] {
@@ -169,6 +179,7 @@ int launch_block_t(qcm_handle h, const BlockArgs &a, size_t smem) {
     kern<<<bgrid(h, grid), kThreads, smem, h->stream>>>(a);
     QCM_CUDA(h, cudaGetLastError());
     h->timing.kernel_launches++;
+    name_kernel(h, "k_block<%s,%d,M=%d,U=%d,LAZY=%d>", real_name<R>(), V, M, U, LAZY ? 1 : 0);
     return QCM_OK;
 }
 
@@ -234,6 +245,7 @@ int launch_expand_t(qcm_handle h, const ExpandArgs &a, size_t smem) {
     kern<<<bgrid(h, grid), threads, smem, h->stream>>>(a);
     QCM_CUDA(h, cudaGetLastError());
     h->timing.kernel_launches++;
+    name_kernel(h, "k_expand<%s,%d,M=%d,U=%d,Q0=%d>", real_name<R>(), V, M, U, Q0 ? 1 : 0);
     return QCM_OK;
 }
 
@@ -614,8 +626,8 @@ int launch_block_plan(qcm_handle h, BlockPlan &bp) {
         h->rot_m = M;
         h->rot_nin = n_in;
     } else if (bp.tree) {
-        h->cur_kernel = h->prec == QCM_C64 ? "k_expand_tree<float>" : "k_expand_tree<double>";
         const int V = (h->prec == QCM_C64 && n_in >= 1) ? 2 : 1;
+        name_kernel(h, "k_expand_tree<%s,%d>", h->prec == QCM_C64 ? "float" : "double", V);
         const int threads = bp.trargs.tree_out ? (1 << kChunkBits) / V : 256;     // fused tree: tile == chunk
         const uint64_t nvec = (1ull << n_in) / V;
         const uint64_t grid = std::min<uint64_t>(std::max<uint64_t>(1, (nvec + threads - 1) / threads), 0x7fffffffull);
@@ -636,7 +648,6 @@ int launch_block_plan(qcm_handle h, BlockPlan &bp) {
         h->timing.kernel_launches++;
         h->n_expand++;
     } else if (bp.expand) {
-        h->cur_kernel = h->prec == QCM_C64 ? "k_expand<float>" : "k_expand<double>";
         const size_t centry = h->prec == QCM_C64 ? 8 : 16;
         const size_t nent = 1ull << (M + bp.targs.nu);
         if ((rc = ensure(h, h->ctab, nent * centry * h->batch))) return rc;
@@ -661,7 +672,6 @@ int launch_block_plan(qcm_handle h, BlockPlan &bp) {
         h->n_expand++;
     } else {
         const bool lazy = n_in != n_out;
-        h->cur_kernel = h->prec == QCM_C64 ? "k_block<float>" : "k_block<double>";
         rc = try_lowq(h, bp);
         if (rc < 0) return rc;
         if (rc == 1) {
@@ -706,14 +716,17 @@ int launch_diag(qcm_handle h, const qcm_op &op, size_t n_tables) {
             auto k = k_diag<float, 2, 4>;
             int grid = (int)std::min<uint64_t>(grid_for(h, k, smem, kThreads * 4, (1ull << a.n_active) / 2), cta_cap);
             k<<<bgrid(h, grid), kThreads, smem, h->stream>>>(a);
+            h->cur_kernel = "k_diag<float,2,U=4>";
         } else {
             auto k = k_diag<float, 1, 4>;
             k<<<bgrid(h, 1), kThreads, smem, h->stream>>>(a);
+            h->cur_kernel = "k_diag<float,1,U=4>";
         }
     } else {
         auto k = k_diag<double, 1, 4>;
         int grid = (int)std::min<uint64_t>(grid_for(h, k, smem, kThreads * 4, 1ull << a.n_active), cta_cap);
         k<<<bgrid(h, grid), kThreads, smem, h->stream>>>(a);
+        h->cur_kernel = "k_diag<double,1,U=4>";
     }
     QCM_CUDA(h, cudaGetLastError());
     h->timing.kernel_launches++;
@@ -788,13 +801,12 @@ int launch_diag_multi(qcm_handle h, const qcm_op *members, int n_mem, int n_acti
                 int rc2 = launch_diag(h, members[k], n_tables);
                 if (rc2) return rc2;
             }
-            h->cur_kernel = "k_diag (diagonal block, one pass per member)";
+            h->cur_kernel += " (diagonal block, one pass per member)";
             return QCM_OK;
         }
     }
     const size_t smem = reals * real_bytes(h);
     if (smem > 200 * 1024) return fail(h, QCM_ERR_UNSUPPORTED, "diagonal block tables need %zu B of shared memory", smem);
-    h->cur_kernel = h->prec == QCM_C64 ? "k_diag_multi<float>" : "k_diag_multi<double>";
     // every CTA stages all tables (up to 16 KiB each): give it at least 16x that much state to sweep, else the
     // staging traffic rivals the state traffic (a 16 MiB sweep point under 32 KiB of tables: 3.3 -> 6+ TB/s)
     const uint64_t cta_cap = std::max<uint64_t>((uint64_t)(4 * h->num_sms + h->batch - 1) / h->batch,
@@ -804,14 +816,17 @@ int launch_diag_multi(qcm_handle h, const qcm_op *members, int n_mem, int n_acti
         auto k = k_diag_multi<float, 2, 4>;
         if (smem > 48 * 1024) QCM_CUDA(h, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         k<<<bgrid(h, capped(grid_for(h, k, smem, kThreads * 4, (1ull << n_active) / 2))), kThreads, smem, h->stream>>>(a, runs);
+        h->cur_kernel = "k_diag_multi<float,2,U=4>";
     } else if (h->prec == QCM_C64) {
         auto k = k_diag_multi<float, 1, 4>;
         if (smem > 48 * 1024) QCM_CUDA(h, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         k<<<bgrid(h, 1), kThreads, smem, h->stream>>>(a, runs);
+        h->cur_kernel = "k_diag_multi<float,1,U=4>";
     } else {
         auto k = k_diag_multi<double, 1, 4>;
         if (smem > 48 * 1024) QCM_CUDA(h, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         k<<<bgrid(h, capped(grid_for(h, k, smem, kThreads * 4, 1ull << n_active))), kThreads, smem, h->stream>>>(a, runs);
+        h->cur_kernel = "k_diag_multi<double,1,U=4>";
     }
     QCM_CUDA(h, cudaGetLastError());
     h->timing.kernel_launches++;
@@ -841,13 +856,16 @@ int launch_init(qcm_handle h, const qcm_op &op, size_t n_tables, const double *h
             auto k = k_init<float, 2>;
             int grid = grid_for(h, k, 0, (uint64_t)kThreads * kInitU, (1ull << n) / 2);
             k<<<bgrid(h, grid), kThreads, 0, h->stream>>>(h->state, h->init_lo.p, (const double2 *)h->init_hi.p, n, L, bst, blo, bhi);
+            h->cur_kernel = "k_init<float,2>";
         } else {
             k_init<float, 1><<<bgrid(h, 1), kThreads, 0, h->stream>>>(h->state, h->init_lo.p, (const double2 *)h->init_hi.p, n, L, bst, blo, bhi);
+            h->cur_kernel = "k_init<float,1>";
         }
     } else {
         auto k = k_init<double, 1>;
         int grid = grid_for(h, k, 0, (uint64_t)kThreads * kInitU, 1ull << n);
         k<<<bgrid(h, grid), kThreads, 0, h->stream>>>(h->state, h->init_lo.p, (const double2 *)h->init_hi.p, n, L, bst, blo, bhi);
+        h->cur_kernel = "k_init<double,1>";
     }
     QCM_CUDA(h, cudaGetLastError());
     h->timing.kernel_launches++;
@@ -884,9 +902,11 @@ int launch_extend(qcm_handle h, int n_in, int n_out) {
     if (h->prec == QCM_C64) {
         auto k = k_zero<float>;
         k<<<bgrid(h, grid_for(h, k, 0, (uint64_t)kThreads * kInitU, count)), kThreads, 0, h->stream>>>(h->state, first, count, bstate(h));
+        h->cur_kernel = "k_zero<float>";
     } else {
         auto k = k_zero<double>;
         k<<<bgrid(h, grid_for(h, k, 0, (uint64_t)kThreads * kInitU, count)), kThreads, 0, h->stream>>>(h->state, first, count, bstate(h));
+        h->cur_kernel = "k_zero<double>";
     }
     QCM_CUDA(h, cudaGetLastError());
     h->timing.kernel_launches++;
@@ -904,13 +924,16 @@ int launch_swap(qcm_handle h, const qcm_op &op) {
         if (qa >= 1 && n >= 3) {
             auto k = k_swap<float, 2>;
             k<<<bgrid(h, grid_for(h, k, 0, kThreads, quads / 2)), kThreads, 0, h->stream>>>(h->state, qa, qb, n, bstate(h));
+            h->cur_kernel = "k_swap<float,2>";
         } else {
             auto k = k_swap<float, 1>;
             k<<<bgrid(h, grid_for(h, k, 0, kThreads, quads)), kThreads, 0, h->stream>>>(h->state, qa, qb, n, bstate(h));
+            h->cur_kernel = "k_swap<float,1>";
         }
     } else {
         auto k = k_swap<double, 1>;
         k<<<bgrid(h, grid_for(h, k, 0, kThreads, quads)), kThreads, 0, h->stream>>>(h->state, qa, qb, n, bstate(h));
+        h->cur_kernel = "k_swap<double,1>";
     }
     QCM_CUDA(h, cudaGetLastError());
     h->timing.kernel_launches++;

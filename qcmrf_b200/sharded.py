@@ -934,15 +934,16 @@ class ShardedSimulator:
         ev = t.cuda.Event()
         ev.record()
         import threading
+        # the record keeps its buffers: a later circuit of another size replaces self._dbuf before this one is collected
         rec = {'event': ev, 'slot': slot, 'nb': nb, 'words': words, 'order': pr.pmf_order, 'done': threading.Event(),
-               'known': known}
+               'known': known, 'bufs': b}
         b['busy'][slot] = rec
         return rec
 
     def _collect_one_collective(self, rec):
         """(keys, probs, kept) of an enqueued record, or None (consistently on every rank) if a measured rank mass
         contradicted the plan -- the caller then takes the general path."""
-        b = self._dbuf
+        b = rec['bufs']
         rec['event'].synchronize()
         nb, words = rec['nb'], rec['words']
         hall = b['h_all'][rec['slot']].numpy().reshape(self.world, words)

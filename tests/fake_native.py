@@ -108,6 +108,8 @@ class Handle:
         return np.arange(1 << self.n_local, dtype=np.int64) | (self.rank << self.n_local)
 
     def postselect(self, mask, value, n_out_bits, want_probs=True, out=None):
+        if not 0 <= n_out_bits <= min(self.n_local, 30):
+            raise RuntimeError('n_out_bits %d out of range' % n_out_bits)        # as qcm_postselect refuses it
         w = np.abs(self.state) ** 2
         w[1 << self.active:] = 0
         idx = self._global_index()

@@ -342,3 +342,80 @@ def test_random_generic_circuits_through_the_public_call(monkeypatch, seed):
             assert 0.5 * np.abs(emp - kp).sum() < bound, (seed, trial, fus, small, width)
             checked += 1
     assert checked >= 16
+
+
+def test_pipelined_list_with_equal_state_size_and_other_pmf_size(monkeypatch):
+    """Two circuits with the same number of stored qubits but different variable counts: the pipeline of run() must
+    collect the first before the second needs result buffers of another size.  Counts, pmf and success probability
+    equal one run() per circuit with the same Philox stream."""
+    import fake_native
+    fake_native.install(monkeypatch)
+    from qcmrf_b200 import B200Simulator
+    rng = np.random.RandomState(12)
+    a = QCMRF([[0, 1], [1, 2], [2, 3], [3, 4]], list(-np.abs(rng.randn(16)) * 0.5))
+    b = QCMRF([[0, 1], [1, 2], [2, 3], [0, 3], [0, 2]], list(-np.abs(rng.randn(20)) * 0.5))
+    sim = B200Simulator(precision='double', small_batch=False, sweep_batch=False, seed=4)
+    assert sim.prepare(a).plan.n_phys == sim.prepare(b).plan.n_phys
+    circs = [a, b, a, b]
+    res = sim.run(circs, shots=1500).result()
+    one = B200Simulator(precision='double', small_batch=False, sweep_batch=False, seed=4)
+    for i, c in enumerate(circs):
+        r1 = one.run(c, shots=1500, stream_ids=[i]).result()
+        assert res.get_counts(i) == r1.get_counts(), i
+        p, d = res.postselected_probabilities(i)
+        p1, d1 = r1.postselected_probabilities(0)
+        assert np.array_equal(p, p1) and d == d1, i
+
+
+def test_sweep_chunks_respect_the_engine_batch_limit(monkeypatch):
+    """A sweep whose points would fit sweep_bytes many times over is still cut into chunks of at most 65 535 points,
+    the most one batched handle takes."""
+    import fake_native
+    fake_native.install(monkeypatch)
+    from qcmrf_b200 import B200Simulator
+    SWEEP_MAX_POINTS = 65535                            # qcm_create_batched refuses more points
+    sim = B200Simulator(precision='single', small_batch=False, seed=1)
+    c = QCMRF([[0, 1], [1, 2]], [-0.3] * 8)
+    pr = sim.prepare(c)
+    n = 70000
+    sim.sweep_bytes = 1 << 40                           # state room for ~2^28 points: only the batch limit applies
+    chunks = []
+
+    class _T:
+        def timing(self):
+            return dict(sample_ms=0.0, postselect_ms=0.0)
+
+    def fake_execute_sweep(sw, shots, seed, streams, precision, pmf, first, B):
+        assert 2 <= B <= SWEEP_MAX_POINTS and len(streams) == B
+        chunks.append((first, B))
+        sim._last = _T()
+        return None, None, np.full(B, 0.5)
+    monkeypatch.setattr(sim, 'execute_sweep', fake_execute_sweep)
+    out = sim._run_sweep([c] * n, [pr] * n, 0, 1, np.arange(n), 'single', False)
+    assert len(out) == n and sum(B for _f, B in chunks) == n
+    assert chunks[0] == (0, SWEEP_MAX_POINTS) and chunks[1] == (SWEEP_MAX_POINTS, n - SWEEP_MAX_POINTS)
+
+
+def test_variables_that_are_never_stored(monkeypatch):
+    """A circuit whose highest variable qubits are never touched stores fewer qubits than it has variables: the
+    large-state path post-selects over the stored ones and pads the pmf with the never-stored qubits' |0>."""
+    import fake_native
+    fake_native.install(monkeypatch)
+    from qcmrf_b200 import B200Simulator
+    from qcmrf_b200.circuit import QuantumCircuit
+    c = QuantumCircuit(4, 4)
+    c.h(0)
+    c.ry(0.7, 1)
+    c.cx(0, 1)
+    c.measure(range(4), range(4))
+    sim = B200Simulator(precision='double', small_batch=False, seed=2)
+    assert sim.prepare(c, n_vars=4).plan.n_phys < 4
+    a = np.array([np.cos(0.35), np.sin(0.35)])
+    want = np.zeros(16)
+    for x0 in (0, 1):
+        for x1 in (0, 1):
+            want[x0 | ((x1 ^ x0) << 1)] = 0.5 * a[x1] ** 2
+    for circs in (c, [c, c]):
+        res = sim.run(circs, shots=500, n_vars=4).result()
+        p, d = res.postselected_probabilities(0)
+        assert np.abs(p - want).max() < 1e-12 and abs(d - 1.0) < 1e-12
