@@ -98,7 +98,12 @@ enum qcm_op_kind {
  * the low address bits, which turns its 2^M write streams into one sequential stream.  Every
  * entry point that reads the state (qcm_postselect*, qcm_sample*, qcm_get_amplitudes) undoes the
  * rotation: callers keep seeing logical indices.  The next program must start with INIT_PRODUCT
- * (or qcm_set_amplitudes); qcm_state_ptr contents are not in logical order until then.        */
+ * (or qcm_set_amplitudes); qcm_state_ptr contents are not in logical order until then.
+ * The result may also be left UNWRITTEN (by default when it has more than 2^30 amplitudes;
+ * QCM_VIRTUAL_LAST in DESIGN.md): the sampler on the QCM_FLAG_SAMPLE_CHECKPOINT tree and the
+ * prefix post-selection compute the amplitudes they read from the pass's input, and every other
+ * reader (general post-selection, qcm_get_amplitudes, a rebuilt sum tree, qcm_state_ptr) first
+ * writes the result out, enqueued on the handle's stream.                                     */
 #define QCM_FLAG_ROTATED_OUTPUT_OK 2
 
 typedef struct qcm_op {

@@ -64,6 +64,12 @@ struct qcm_sim_s {
     // physical address ((i & (2^rot_nin - 1)) << rot_m) | (i >> rot_nin); rot_m == 0: identity
     int rot_m = 0, rot_nin = 0;
     bool tree_cond_low = false;     // the checkpoint tree's conditional images are the low address bits
+    // virtual last pass (QCM_VIRTUAL_LAST): the rotated result was left unwritten.  Its input stays in `scratch`, and
+    // readers compute the images they need from it with these arguments (low_image); materialise_last() writes it
+    // out for the readers that need the state itself.
+    bool virt = false;
+    ExpandTreeArgs virt_args{};
+    size_t virt_smem = 0;
     std::vector<double> h_top;
     // sum tree (built by qcm_sample_prepare)
     int tree_levels = 0;
@@ -274,6 +280,7 @@ struct BlockPlan {
     bool norm_preserving = false;   // expansion without diagonal members: sum_a |out[x,a]|^2 == |in[x]|^2
     bool rotate = false;            // store the result rotated (k_expand_low); decided by the program loop
     bool input_in_scratch = false;  // ... and its input already lives in h->scratch (the program prefix ran there)
+    bool virt = false;              // ... and is left unwritten: only the checkpoint sums run (see qcm_sim_s::virt)
 };
 
 // members: ops[0..n_mem) are MUX1Q (or DIAG: a diagonal factor applied in the same sweep);
@@ -450,12 +457,39 @@ int low_ctas() {
     return v;
 }
 
-template <typename R, int V, int MH, int TB, int NW>
+// QCM_VIRTUAL_LAST = 0: always write the rotated last pass; 1: leave it unwritten (virtual) at any size; unset: leave it
+// unwritten when its output has more than 2^30 amplitudes -- the rotated states qcm_get_amplitudes never returned.
+int virtual_last() {
+    static int v = [] {
+        const char *e = getenv("QCM_VIRTUAL_LAST");
+        return (e && (e[0] == '0' || e[0] == '1')) ? e[0] - '0' : -1;
+    }();
+    return v;
+}
+
+// Raises a kernel's dynamic shared-memory limit to the device's opt-in maximum, once per kernel and device, before its
+// first launch there.  Changing a function's attributes while an instance of it runs holds the call back until that
+// instance ends (another rank's kernel on this GPU waiting for signals, or this stream's previous pass), and handles
+// that share a process get here concurrently, so the check and the set happen under one lock.
+int raise_smem_limit(qcm_handle h, const void *kern) {
+    static std::mutex mu;
+    static std::set<std::pair<int, const void *>> done;
+    std::lock_guard<std::mutex> lock(mu);
+    if (done.count({h->device, kern})) return QCM_OK;
+    int optin = 0;
+    QCM_CUDA(h, cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+    QCM_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
+    done.insert({h->device, kern});
+    return QCM_OK;
+}
+
+// EMIT = false: the sums-only launch of a virtual last pass (no tables, no stores of the state)
+template <typename R, int V, int MH, int TB, int NW, bool EMIT>
 static int launch_low_tb(qcm_handle h, int n_in, BlockPlan &bp) {
-    auto kern = k_expand_low<R, V, MH, TB, NW>;
+    auto kern = k_expand_low<R, V, MH, TB, NW, EMIT>;
     constexpr int warps = NW;
-    size_t smem = low_warp_bytes<R, MH>() * warps + bp.tree_smem;
-    {
+    size_t smem = EMIT ? low_warp_bytes<R, MH>() * warps + bp.tree_smem : 0;
+    if (EMIT) {
         // default: 24 resident warps per SM for complex64 (q34 last pass, profiles/r02_low_ctas_sweep.txt: 8x8 at 5 / 4 / 3 /
         // 2 CTAs per SM 9.72 / 9.67 / 9.65 / 10.02 ms, 4x7 at 10 / 8 / 6 / 5 / 4: 9.78 / 9.72 / 9.66 / 9.74 / 10.00);
         // complex128 CTAs (4 warps, twice the shared memory) already sit at 6 per SM
@@ -465,18 +499,20 @@ static int launch_low_tb(qcm_handle h, int n_in, BlockPlan &bp) {
             if (per_cta > smem) smem = per_cta;
         }
     }
-    if (smem > 48 * 1024) QCM_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int rc;
+    if (smem > 48 * 1024 && (rc = raise_smem_limit(h, (const void *)kern))) return rc;
     ExpandTreeArgs args = bp.trargs;
     double *level0 = args.tree_out;
     if (level0) {                                          // per-warp partial sums, grouped into level 0 below
-        int rc = ensure(h, h->lowpart, (sizeof(double) * warps) << (n_in - TB));
+        rc = ensure(h, h->lowpart, (sizeof(double) * warps) << (n_in - TB));
         if (rc) return rc;
         args.tree_out = (double *)h->lowpart.p;
     }
     kern<<<1u << (n_in - TB), NW * 32, smem, h->stream>>>(args, h->scratch.p);
     {
         char nm[96];
-        snprintf(nm, sizeof nm, "k_expand_low<%s,%d,MH=%d,TB=%d,NW=%d>", sizeof(R) == 4 ? "float" : "double", V, MH, TB, NW);
+        if (EMIT) snprintf(nm, sizeof nm, "k_expand_low<%s,%d,MH=%d,TB=%d,NW=%d>", sizeof(R) == 4 ? "float" : "double", V, MH, TB, NW);
+        else snprintf(nm, sizeof nm, "k_expand_low_sums<%s,%d,TB=%d,NW=%d>", sizeof(R) == 4 ? "float" : "double", V, TB, NW);
         h->cur_kernel = nm;
     }
     QCM_CUDA(h, cudaGetLastError());
@@ -491,16 +527,16 @@ static int launch_low_tb(qcm_handle h, int n_in, BlockPlan &bp) {
     return QCM_OK;
 }
 
-template <typename R, int V, int MH>
+template <typename R, int V, int MH, bool EMIT = true>
 static int launch_low(qcm_handle h, int n_in, BlockPlan &bp) {
     // complex128 CTAs have always been 4 warps (twice the shared memory per warp)
     const int shape = (sizeof(R) == 8 && low_shape() == 808) ? 407 : low_shape();
     switch (shape) {
-        case 810: return launch_low_tb<R, V, MH, 10, 8>(h, n_in, bp);
-        case 407: return launch_low_tb<R, V, MH, 7, 4>(h, n_in, bp);
-        case 206: return launch_low_tb<R, V, MH, 6, 2>(h, n_in, bp);
-        case 105: return launch_low_tb<R, V, MH, 5, 1>(h, n_in, bp);
-        default: return launch_low_tb<R, V, MH, 8, 8>(h, n_in, bp);
+        case 810: return launch_low_tb<R, V, MH, 10, 8, EMIT>(h, n_in, bp);
+        case 407: return launch_low_tb<R, V, MH, 7, 4, EMIT>(h, n_in, bp);
+        case 206: return launch_low_tb<R, V, MH, 6, 2, EMIT>(h, n_in, bp);
+        case 105: return launch_low_tb<R, V, MH, 5, 1, EMIT>(h, n_in, bp);
+        default: return launch_low_tb<R, V, MH, 8, 8, EMIT>(h, n_in, bp);
     }
 }
 
@@ -617,14 +653,30 @@ int launch_block_plan(qcm_handle h, BlockPlan &bp) {
             h->timing.bytes_read += in_bytes;      // the scratch copy: one more read and write of the input
             h->timing.bytes_written += in_bytes;
         }
-        if (h->prec == QCM_C64) rc = launch_low_mh<float, 2>(h, M - 6, n_in, bp);
+        // a virtual pass runs the checkpoint sums only, in the materialising launch's shape (the same level-0
+        // association), and nothing at all without the checkpoint
+        const bool launch = !bp.virt || bp.trargs.tree_out;
+        if (!launch) rc = QCM_OK;
+        else if (bp.virt) rc = h->prec == QCM_C64 ? launch_low<float, 2, 0, false>(h, n_in, bp) : launch_low<double, 1, 0, false>(h, n_in, bp);
+        else if (h->prec == QCM_C64) rc = launch_low_mh<float, 2>(h, M - 6, n_in, bp);
         else rc = launch_low_mh<double, 1>(h, M - 5, n_in, bp);
         if (rc) return rc;
         QCM_CUDA(h, cudaGetLastError());
-        h->timing.kernel_launches++;
+        if (launch) h->timing.kernel_launches++;
         h->n_expand++;
         h->rot_m = M;
         h->rot_nin = n_in;
+        if (bp.virt) {
+            h->virt = true;
+            h->virt_args = bp.trargs;
+            h->virt_args.tree_out = nullptr;     // materialise_last: the tree exists already
+            h->virt_smem = bp.tree_smem;
+            if (launch) {                        // algorithmic traffic: the input read, the finer sum level written
+                h->timing.bytes_read += in_bytes;
+                h->timing.bytes_written += sizeof(double) << (n_in - (h->prec == QCM_C64 ? 1 : 0));
+            }
+            return QCM_OK;
+        }
     } else if (bp.tree) {
         const int V = (h->prec == QCM_C64 && n_in >= 1) ? 2 : 1;
         name_kernel(h, "k_expand_tree<%s,%d>", h->prec == QCM_C64 ? "float" : "double", V);
@@ -688,6 +740,23 @@ int launch_block_plan(qcm_handle h, BlockPlan &bp) {
     // algorithmic traffic: read the materialised input, write the whole output
     h->timing.bytes_read += amp_bytes(h->prec) << n_in;
     h->timing.bytes_written += amp_bytes(h->prec) << n_out;
+    return QCM_OK;
+}
+
+// Writes out the unwritten result of a virtual last pass (qcm_sim_s::virt), from its input, for the readers that need
+// the state itself.  Enqueued on the handle's stream; a no-op for any other state.
+int materialise_last(qcm_handle h) {
+    if (!h->virt) return QCM_OK;
+    h->virt = false;
+    BlockPlan bp;
+    bp.trargs = h->virt_args;
+    bp.tree_smem = h->virt_smem;
+    const int M = bp.trargs.M, n_in = bp.trargs.n_in;
+    const std::string kernel = h->cur_kernel;            // not an op of a program: leave the per-op record alone
+    int rc = h->prec == QCM_C64 ? launch_low_mh<float, 2>(h, M - 6, n_in, bp) : launch_low_mh<double, 1>(h, M - 5, n_in, bp);
+    h->cur_kernel = kernel;
+    if (rc) return rc;
+    h->timing.kernel_launches++;
     return QCM_OK;
 }
 
@@ -1061,6 +1130,7 @@ int tree_finish(qcm_handle h, int na) {
 int build_tree(qcm_handle h) {
     const int na = h->n_active;
     int rc;
+    if ((rc = materialise_last(h))) return rc;
     if ((rc = tree_layout(h, na))) return rc;
     if ((rc = tree_level0(h, na))) return rc;
     return tree_finish(h, na);
@@ -1144,21 +1214,9 @@ static int launch_gather_inplace(qcm_handle h, const GatherArgs &a, const Gather
     auto kern = k_block_gather_inplace<R, V, M, 1, S>;
     const size_t smem = 256 + (size_t)S * (1 << M) * kGatherTileBytes + tab_bytes;
     if (smem > 227 * 1024) return fail(h, QCM_ERR_UNSUPPORTED, "gather ring needs %zu B of shared memory", smem);
-    // set once per kernel and device, to the most any launch may ask for, before the first launch: changing a function's
-    // attributes while an instance of it is running (another rank's kernel on this GPU, already waiting for signals) would
-    // hold this launch back until that instance ends.  Ranks that share a process (threads, one handle each) get here
-    // concurrently, so the check and the set happen under one lock.
-    static std::mutex attr_mu;
-    static std::set<int> attr_set;
-    {
-        std::lock_guard<std::mutex> lock(attr_mu);
-        if (!attr_set.count(h->device)) {
-            int optin = 0;
-            QCM_CUDA(h, cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
-            QCM_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
-            attr_set.insert(h->device);
-        }
-    }
+    // set once, before the first launch: another rank's instance may already be waiting for signals (raise_smem_limit)
+    int rc;
+    if ((rc = raise_smem_limit(h, (const void *)kern))) return rc;
     const uint64_t tiles = ((1ull << (a.n_local - M)) / V) / kThreads;
     int K = env_int("QCM_GATHER_K", 16);
     int p2 = 1;
@@ -1356,6 +1414,7 @@ int qcm_get_amplitudes(qcm_handle h, uint64_t first, uint64_t count, void *host_
     if (h->rot_m && first < vend) {
         // rotated storage: fetch the active state and undo the rotation on the host (inspection path)
         if (h->n_active > 30) return fail(h, QCM_ERR_UNSUPPORTED, "qcm_get_amplitudes on a rotated state of %d qubits", h->n_active);
+        if ((rc = materialise_last(h))) return rc;
         std::vector<char> tmp((size_t)valid * ab);
         QCM_CUDA(h, cudaMemcpyAsync(tmp.data(), st, (size_t)valid * ab, cudaMemcpyDeviceToHost, h->stream));
         QCM_CUDA(h, cudaStreamSynchronize(h->stream));
@@ -1387,11 +1446,15 @@ int qcm_set_amplitudes(qcm_handle h, uint64_t first, uint64_t count, const void 
     h->tree_valid = false;
     h->product_n = -1;
     h->rot_m = h->rot_nin = 0;
+    h->virt = false;
     return QCM_OK;
 }
 
 int qcm_state_ptr(qcm_handle h, void **dev_ptr_out, uint64_t *bytes_out) {
     if (!h) return fail(nullptr, QCM_ERR_INVALID, "handle is NULL");
+    int rc = check_device(h);
+    if (rc) return rc;
+    if ((rc = materialise_last(h))) return rc;
     if (dev_ptr_out) *dev_ptr_out = h->state;
     if (bytes_out) *bytes_out = (amp_bytes(h->prec) << h->n_local) * (uint64_t)h->batch;
     return QCM_OK;
@@ -1481,6 +1544,12 @@ int qcm_run_program(qcm_handle h, const qcm_op *ops, int n_ops, const double *ta
     if (rc) return rc;
     h->tree_valid = false;
     h->product_n = -1;
+    if (h->virt) {
+        // the unwritten result depends on this handle's tables and scratch buffer, which this program may reuse: a new
+        // state drops it, anything else (which is refused below) writes it out first
+        if (n_ops > 0 && ops[0].kind == QCM_OP_INIT_PRODUCT) h->virt = false;
+        else if ((rc = materialise_last(h))) return rc;
+    }
     bool keep_tree = false;
     h->timing.bytes_read = h->timing.bytes_written = 0;
     QCM_CUDA(h, cudaEventRecord(h->ev0, h->stream));
@@ -1589,6 +1658,10 @@ int qcm_run_program(qcm_handle h, const qcm_op *ops, int n_ops, const double *ta
                     cudaGetLastError();                   // no room for the input copy: keep the in-place kernel
                     bp.rotate = false;
                 }
+                // virtual: the result is left unwritten, its readers compute the images they use from the input (the
+                // sampler on the checkpoint tree: one leaf's images per shot, the prefix post-selection: image 0 of
+                // each kept input); without the checkpoint a sampler rebuilds the tree and writes the result out first
+                bp.virt = bp.rotate && (virtual_last() == 1 || (virtual_last() < 0 && op.n_active_out > 30));
                 bp.input_in_scratch = input_in_scratch;
                 if (input_in_scratch && !bp.rotate) {     // the prefix ran in the scratch buffer after all: bring it home
                     QCM_CUDA(h, cudaMemcpyAsync(h->state, h->scratch.p, amp_bytes(h->prec) << op.n_active_in,
@@ -1846,9 +1919,17 @@ static int postselect_impl(qcm_handle h, uint64_t mask, uint64_t value, int n_ou
         if (contiguous && (!h->rot_m || pshift)) {
             const uint64_t count = 1ull << nb;
             if (dprobs && count < nprob) QCM_CUDA(h, cudaMemsetAsync(dprobs, 0, nprob * B * sizeof(double), h->stream));
-            if (h->prec == QCM_C64) k_probs_prefix<float><<<bgrid(h, blocks), kThreads, 0, h->stream>>>(h->state, count, pshift, dprobs, (double *)h->partial.p, bstate(h), bprobs, bpart);
-            else k_probs_prefix<double><<<bgrid(h, blocks), kThreads, 0, h->stream>>>(h->state, count, pshift, dprobs, (double *)h->partial.p, bstate(h), bprobs, bpart);
+            double *const part = (double *)h->partial.p;
+            if (h->virt) {                        // image 0 of each kept input, from the unwritten pass's input
+                if (h->prec == QCM_C64) k_probs_prefix<float, true><<<bgrid(h, blocks), kThreads, 0, h->stream>>>(h->scratch.p, count, 0, dprobs, part, 0, bprobs, bpart, h->virt_args);
+                else k_probs_prefix<double, true><<<bgrid(h, blocks), kThreads, 0, h->stream>>>(h->scratch.p, count, 0, dprobs, part, 0, bprobs, bpart, h->virt_args);
+            } else if (h->prec == QCM_C64) {
+                k_probs_prefix<float, false><<<bgrid(h, blocks), kThreads, 0, h->stream>>>(h->state, count, pshift, dprobs, part, bstate(h), bprobs, bpart, ExpandTreeArgs{});
+            } else {
+                k_probs_prefix<double, false><<<bgrid(h, blocks), kThreads, 0, h->stream>>>(h->state, count, pshift, dprobs, part, bstate(h), bprobs, bpart, ExpandTreeArgs{});
+            }
         } else {
+            if ((rc = materialise_last(h))) return rc;
             if (dprobs) QCM_CUDA(h, cudaMemsetAsync(dprobs, 0, nprob * B * sizeof(double), h->stream));
             if (h->prec == QCM_C64)
                 k_postselect_general<float><<<bgrid(h, blocks), kThreads, 0, h->stream>>>(h->state, h->n_active, rb, mask, value, nprob - 1, h->rot_m, h->rot_nin, dprobs, (double *)h->partial.p, bstate(h), bprobs, bpart);
@@ -1985,6 +2066,10 @@ static int sample_sharded_impl(qcm_handle h, uint64_t shots, uint64_t seed, uint
     a.cond_low = (h->tree_cond_bits && h->tree_cond_low) ? 1 : 0;
     a.rot_m = h->rot_m;
     a.rot_nin = h->rot_nin;
+    if (h->virt) {                           // the tree is the virtual pass's checkpoint (a rebuilt one materialised it)
+        a.virt_in = h->scratch.p;
+        a.virt = h->virt_args;
+    }
     a.sub = (h->tree_has_sub || h->tree_sub_strided) ? (const double *)h->subtree.p : nullptr;
     a.sub_bits = h->tree_sub_bits;
     a.sub_strided = (h->tree_sub_strided && !h->tree_has_sub) ? 1 : 0;

@@ -1292,6 +1292,102 @@ template <typename R, int MH> __host__ __device__ constexpr size_t low_warp_byte
 // small CTAs (8 / 4 warps): five or more resident per SM, so one CTA's start-up (table staging) overlaps the others' stores
 template <typename R> __host__ __device__ constexpr int low_threads() { return sizeof(R) == 4 ? 256 : 128; }
 
+// ---- the image arithmetic of the rotated pass, shared by k_expand_low and by the readers of an unwritten (virtual)
+// result, which compute the images they need from the pass's input instead of loading them (DESIGN.md 3).  Every
+// complex multiply is written with explicit roundings, so the FMA contraction cannot differ between the kernel and a
+// reader: a computed image is bit-identical to the stored one.  fac(member, bit, fr, fi) yields f_member[bit] at the
+// input's table index.
+__device__ __forceinline__ void low_cmul(float ar, float ai, float br, float bi, float &cr, float &ci) {
+    const float t = __fmul_rn(ai, bi), u = __fmul_rn(ai, br);
+    cr = __fmaf_rn(ar, br, -t);
+    ci = __fmaf_rn(ar, bi, u);
+}
+__device__ __forceinline__ void low_cmul(double ar, double ai, double br, double bi, double &cr, double &ci) {
+    const double t = __dmul_rn(ai, bi), u = __dmul_rn(ai, br);
+    cr = __fma_rn(ar, br, -t);
+    ci = __fma_rn(ar, bi, u);
+}
+// table index of member m at global index gi
+__device__ __forceinline__ uint32_t low_index(const TreeMember &m, uint64_t gi) {
+    uint32_t idx = 0;
+#pragma unroll 1
+    for (int j = 0; j < m.n_ctrl; ++j) idx |= (uint32_t)((gi >> m.ctrl[j]) & 1ull) << j;
+    return idx;
+}
+// p = in[x] * prod_d diag_d[idx_d(x)]; diag(d, idx) points at the real part of entry idx of diagonal d
+template <typename R, typename D>
+__device__ __forceinline__ void low_diag(const ExpandTreeArgs &a, uint64_t gi, D diag, R &pr, R &pi) {
+#pragma unroll 1
+    for (int d = 0; d < a.n_diag; ++d) {
+        const R *c = diag(d, low_index(a.diag[d], gi));
+        low_cmul(pr, pi, c[0], c[1], pr, pi);
+    }
+}
+// q[v] = p * f_0[v] (complex64: member 0 is the vector slot), or p itself
+template <typename R, int V, typename F>
+__device__ __forceinline__ void low_q(F fac, R pr, R pi, int v, R &qr, R &qi) {
+    if constexpr (V == 2) {
+        R fr, fi;
+        fac(0, v, fr, fi);
+        low_cmul(pr, pi, fr, fi, qr, qi);
+    } else {
+        qr = pr; qi = pi;
+    }
+}
+// g[s] = prod_{l < mh} f_{lb + l}[s_l], from 1
+template <typename R, typename F>
+__device__ __forceinline__ void low_g(F fac, int lb, int mh, uint32_t s, R &gr, R &gi) {
+    gr = R(1); gi = R(0);
+#pragma unroll
+    for (int l = 0; l < mh; ++l) {
+        R fr, fi;
+        fac(lb + l, (s >> l) & 1, fr, fi);
+        low_cmul(gr, gi, fr, fi, gr, gi);
+    }
+}
+// A[t] = f_{j0}[t_0] f_{j0+1}[t_1],  B[t] = f_{j0+2}[t_0] f_{j0+3}[t_1] f_{j0+4}[t_2]
+template <typename R, typename F>
+__device__ __forceinline__ void low_a(F fac, int j0, int t, R &cr, R &ci) {
+    R xr, xi, yr, yi;
+    fac(j0, t & 1, xr, xi);
+    fac(j0 + 1, t >> 1, yr, yi);
+    low_cmul(xr, xi, yr, yi, cr, ci);
+}
+template <typename R, typename F>
+__device__ __forceinline__ void low_b(F fac, int j0, int t, R &cr, R &ci) {
+    R xr, xi, yr, yi, zr, zi;
+    fac(j0 + 2, t & 1, xr, xi);
+    fac(j0 + 3, (t >> 1) & 1, yr, yi);
+    fac(j0 + 4, t >> 2, zr, zi);
+    low_cmul(xr, xi, yr, yi, xr, xi);
+    low_cmul(xr, xi, zr, zi, cr, ci);
+}
+// image im (0 <= im < 2^M) of the input with diagonal product p: the amplitude k_expand_low stores at (x << M) | im,
+// L * U[s][v] with im = v | lane << (V - 1) | s << LB and lane = ta | tb << 2, L = A[ta] B[tb]
+template <typename R, int V, typename F>
+__device__ __forceinline__ void low_image(F fac, int M, R pr, R pi, uint32_t im, R &outr, R &outi) {
+    constexpr int LB = V == 2 ? 6 : 5, J0 = V == 2 ? 1 : 0;
+    const uint32_t lane = (im >> (V - 1)) & 31u;
+    R qr, qi, gr, gi, ur, ui, ar, ai, br, bi, lr, li;
+    low_q<R, V>(fac, pr, pi, (int)(im & 1u), qr, qi);
+    low_g<R>(fac, LB, M - LB, im >> LB, gr, gi);
+    low_cmul(qr, qi, gr, gi, ur, ui);
+    low_a<R>(fac, J0, (int)(lane & 3u), ar, ai);
+    low_b<R>(fac, J0, (int)(lane >> 2), br, bi);
+    low_cmul(ar, ai, br, bi, lr, li);
+    low_cmul(lr, li, ur, ui, outr, outi);
+}
+// f_member[bit] read from the program's tables (8 reals per index, column 0 of each 2x2: m00 at 0, m10 at 4)
+template <typename R>
+__device__ __forceinline__ void low_fac_global(const ExpandTreeArgs &a, int member, uint64_t gi, int bit, R &fr, R &fi) {
+    const R *f = reinterpret_cast<const R *>(a.tables) + a.mem[member].src_off + 8 * low_index(a.mem[member], gi) + 4 * bit;
+    fr = f[0]; fi = f[1];
+}
+template <typename R>
+__device__ __forceinline__ const R *low_diag_global(const ExpandTreeArgs &a, int d, uint32_t idx) {
+    return reinterpret_cast<const R *>(a.tables) + a.diag[d].src_off + 2 * idx;
+}
+
 // out[j] = sum of the 2^gbits consecutive values in[j << gbits ...], in index order (deterministic)
 static __global__ void __launch_bounds__(kThreads) k_group_sum(const double *in, int gbits, uint64_t n_out, double *out) {
     const uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1307,7 +1403,9 @@ static __global__ void __launch_bounds__(kThreads) k_group_sum(const double *in,
 // NW: warps per CTA.  The size of the region a CTA writes decides how compact the window of concurrently written addresses
 // is (tools/membench4.cu, profiles/r02_notes.md: a bare sequential writer loses 5 % going from 32 KiB to 512 KiB per CTA),
 // so small CTAs -- few warps, one batch of 32 inputs each -- are the default shape.
-template <typename R, int V, int MH, int TB, int NW = low_threads<R>() / 32>
+// EMIT = false: the sums only (input load, sub_out, level 0) -- the result is left unwritten and its readers compute the
+// images they need (the virtual last pass, DESIGN.md 3); same TB / NW as the materialising launch, so the same tree.
+template <typename R, int V, int MH, int TB, int NW = low_threads<R>() / 32, bool EMIT = true>
 __global__ void __launch_bounds__(NW * 32) k_expand_low(const __grid_constant__ ExpandTreeArgs a, const void *__restrict__ in) {
     constexpr int LB = V == 2 ? 6 : 5;                   // image bits covered by one warp store
     constexpr int J0 = V == 2 ? 1 : 0;                   // first lane-indexed member (member 0 is the vector slot for V == 2)
@@ -1332,30 +1430,25 @@ __global__ void __launch_bounds__(NW * 32) k_expand_low(const __grid_constant__ 
     };
     // the first input amplitude is requested before anything else (its DRAM latency then overlaps the table staging)
     C2 next_in = in_at(x_first(0), 2 * kWarps);
-    for (int j = 0; j < M; ++j) {                         // column 0 of every 2x2: (m00, m10)
-        const int n = 1 << a.mem[j].n_ctrl;
-        for (int i = threadIdx.x; i < n; i += blockDim.x) {
-            const R *src = gt + a.mem[j].src_off + 8 * i;
-            R *dst = tab + a.mem[j].tab_off + 4 * i;
-            dst[0] = src[0]; dst[1] = src[1]; dst[2] = src[4]; dst[3] = src[5];
+    if constexpr (EMIT) {
+        for (int j = 0; j < M; ++j) {                     // column 0 of every 2x2: (m00, m10)
+            const int n = 1 << a.mem[j].n_ctrl;
+            for (int i = threadIdx.x; i < n; i += blockDim.x) {
+                const R *src = gt + a.mem[j].src_off + 8 * i;
+                R *dst = tab + a.mem[j].tab_off + 4 * i;
+                dst[0] = src[0]; dst[1] = src[1]; dst[2] = src[4]; dst[3] = src[5];
+            }
         }
+        for (int d = 0; d < a.n_diag; ++d) {
+            const int n = 2 << a.diag[d].n_ctrl;
+            for (int i = threadIdx.x; i < n; i += blockDim.x) tab[a.diag[d].tab_off + i] = gt[a.diag[d].src_off + i];
+        }
+        __syncthreads();                                  // the only block-level barrier: member tables staged
     }
-    for (int d = 0; d < a.n_diag; ++d) {
-        const int n = 2 << a.diag[d].n_ctrl;
-        for (int i = threadIdx.x; i < n; i += blockDim.x) tab[a.diag[d].tab_off + i] = gt[a.diag[d].src_off + i];
-    }
-    __syncthreads();                                      // the only block-level barrier: member tables staged
     unsigned char *wbase = smem_raw + low_warp_bytes<R, MH>() * warp;
     V16 *Us = reinterpret_cast<V16 *>(wbase);                                      // [NS][32]
     C2 *As = reinterpret_cast<C2 *>(wbase + (size_t)NS * 32 * 16);                 // [4][kLowRow]: a lane reads row lane & 3
     C2 *Bs = As + 4 * kLowRow;                                                     // [8][kLowRow]: a lane reads row lane >> 2
-    auto index_of = [&](const TreeMember &m, uint64_t gi) -> uint32_t {
-        uint32_t idx = 0;
-#pragma unroll 1
-        for (int j = 0; j < m.n_ctrl; ++j) idx |= (uint32_t)((gi >> m.ctrl[j]) & 1ull) << j;
-        return idx;
-    };
-    auto cmul = [](R ar, R ai, R br, R bi, R &cr, R &ci) { cr = ar * br - ai * bi; ci = ar * bi + ai * br; };
     const C2 *my_a = As + (lane & 3) * kLowRow, *my_b = Bs + (lane >> 2) * kLowRow;
 
     // one batch of 32 inputs x0 + (i >> 1) * pstride + (i & 1), i = 0..31; `mine` is lane's input amplitude
@@ -1375,66 +1468,42 @@ __global__ void __launch_bounds__(NW * 32) k_expand_low(const __grid_constant__ 
                 }
                 wacc += w;
             }
+            if constexpr (!EMIT) return;
             R pr = mine.x, pi = mine.y;
-#pragma unroll 1
-            for (int d = 0; d < a.n_diag; ++d) {
-                const uint32_t idx = index_of(a.diag[d], gi);
-                cmul(pr, pi, tab[a.diag[d].tab_off + 2 * idx], tab[a.diag[d].tab_off + 2 * idx + 1], pr, pi);
-            }
+            low_diag(a, gi, [&](int d, uint32_t idx) { return tab + a.diag[d].tab_off + 2 * idx; }, pr, pi);
             __syncwarp();                                 // the previous batch's phase B is done with the tables
             uint32_t off[M];                              // table offset (reals) of member j at this input's index
 #pragma unroll
-            for (int j = 0; j < M; ++j) off[j] = (uint32_t)a.mem[j].tab_off + 4u * index_of(a.mem[j], gi);
+            for (int j = 0; j < M; ++j) off[j] = (uint32_t)a.mem[j].tab_off + 4u * low_index(a.mem[j], gi);
             auto fac = [&](int member, int bit, R &fr, R &fi) {          // f_member[bit] at this input's table index
                 const C2 f = *reinterpret_cast<const C2 *>(tab + off[member] + 2 * bit);
                 fr = f.x; fi = f.y;
             };
             // U[s][v] = in * diag * f_0[v] * prod_{l < MH} f_{LB+l}[s_l]
             R qr[V], qi[V];
-            if constexpr (V == 2) {
 #pragma unroll
-                for (int v = 0; v < 2; ++v) {
-                    R fr, fi;
-                    fac(0, v, fr, fi);
-                    cmul(pr, pi, fr, fi, qr[v], qi[v]);
-                }
-            } else {
-                qr[0] = pr; qi[0] = pi;
-            }
+            for (int v = 0; v < V; ++v) low_q<R, V>(fac, pr, pi, v, qr[v], qi[v]);
 #pragma unroll
             for (int s = 0; s < NS; ++s) {
-                R gr = R(1), gim = R(0);
-#pragma unroll
-                for (int l = 0; l < MH; ++l) {
-                    R fr, fi;
-                    fac(LB + l, (s >> l) & 1, fr, fi);
-                    cmul(gr, gim, fr, fi, gr, gim);
-                }
+                R gr, gim;
+                low_g<R>(fac, LB, MH, s, gr, gim);
                 R ur[V], ui[V];
 #pragma unroll
-                for (int v = 0; v < V; ++v) cmul(qr[v], qi[v], gr, gim, ur[v], ui[v]);
+                for (int v = 0; v < V; ++v) low_cmul(qr[v], qi[v], gr, gim, ur[v], ui[v]);
                 if constexpr (V == 2) Us[s * 32 + lane] = make_float4(ur[0], ui[0], ur[1], ui[1]);
                 else Us[s * 32 + lane] = make_double2(ur[0], ui[0]);
             }
             // A[a] = f_{J0}[a_0] f_{J0+1}[a_1],  B[b] = f_{J0+2}[b_0] f_{J0+3}[b_1] f_{J0+4}[b_2]  (lane = a | b << 2)
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
-                R xr, xi, yr, yi;
-                fac(J0, t & 1, xr, xi);
-                fac(J0 + 1, t >> 1, yr, yi);
                 C2 o;
-                cmul(xr, xi, yr, yi, o.x, o.y);
+                low_a<R>(fac, J0, t, o.x, o.y);
                 As[t * kLowRow + lane] = o;
             }
 #pragma unroll
             for (int t = 0; t < 8; ++t) {
-                R xr, xi, yr, yi, zr, zi;
-                fac(J0 + 2, t & 1, xr, xi);
-                fac(J0 + 3, (t >> 1) & 1, yr, yi);
-                fac(J0 + 4, t >> 2, zr, zi);
-                cmul(xr, xi, yr, yi, xr, xi);
                 C2 o;
-                cmul(xr, xi, zr, zi, o.x, o.y);
+                low_b<R>(fac, J0, t, o.x, o.y);
                 Bs[t * kLowRow + lane] = o;
             }
             __syncwarp();
@@ -1444,17 +1513,17 @@ __global__ void __launch_bounds__(NW * 32) k_expand_low(const __grid_constant__ 
         for (int i = 0; i < 32; ++i) {
             const C2 fa = my_a[i], fb = my_b[i];
             R lr, li;
-            cmul(fa.x, fa.y, fb.x, fb.y, lr, li);
+            low_cmul(fa.x, fa.y, fb.x, fb.y, lr, li);
             const uint64_t obase = (x_of(i) << M) + (uint64_t)lane * V;
 #pragma unroll
             for (int s = 0; s < NS; ++s) {
                 const V16 u = Us[s * 32 + i];
                 R orr[V], oi[V];
                 if constexpr (V == 2) {
-                    cmul(lr, li, u.x, u.y, orr[0], oi[0]);
-                    cmul(lr, li, u.z, u.w, orr[1], oi[1]);
+                    low_cmul(lr, li, u.x, u.y, orr[0], oi[0]);
+                    low_cmul(lr, li, u.z, u.w, orr[1], oi[1]);
                 } else {
-                    cmul(lr, li, u.x, u.y, orr[0], oi[0]);
+                    low_cmul(lr, li, u.x, u.y, orr[0], oi[0]);
                 }
                 VecIO<R, V>::store(a.state, obase + ((uint64_t)s << LB), orr, oi);
             }
@@ -1908,10 +1977,19 @@ struct SampleArgs {
     const double *dev_masses;
     int64_t mass_stride;
     int32_t n_ranks, my_rank;
+    // cond_low with the rotated pass left unwritten: its input (virt_in, 2^n_active amplitudes) and its arguments;
+    // the leaf's images are computed (low_image) instead of loaded
+    const void *virt_in;
+    ExpandTreeArgs virt;
 };
 
 template <typename R>
 __global__ void __launch_bounds__(kThreads) k_sample(const __grid_constant__ SampleArgs a) {
+    using C2 = typename CplxOf<R>::T;
+    // virtual leaf: f_j[bit] of each of the leaf's inputs (at most 2: the finer level sums input pairs) and their
+    // diagonal products, worked out once per shot
+    __shared__ C2 s_vf[kThreads / 32][2][QCM_MAX_EXPAND][2];
+    __shared__ C2 s_vp[kThreads / 32][2];
     const int lane = threadIdx.x & 31;
     const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const uint64_t nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
@@ -2004,7 +2082,37 @@ __global__ void __launch_bounds__(kThreads) k_sample(const __grid_constant__ Sam
         // leaf: the remaining x's, each with its 2^cond_bits images -- one flat, lane-strided search over
         // the (x, image) pairs (image-major, so that consecutive lanes read consecutive amplitudes)
         uint64_t within;
-        if (a.cond_low) {
+        if (a.cond_low && a.virt_in) {
+            // rotated expansion, left unwritten: the same flat search, over computed images
+            const int wl = threadIdx.x >> 5;
+            const uint32_t k = (uint32_t)lane >> 4, j = ((uint32_t)lane >> 1) & 7u;
+            const uint64_t gi = (afirst + k) | a.rank_bits;
+            __syncwarp();                                 // the previous shot is done with the factors
+            if (k < leaf_cnt && (int)j < a.virt.M) {
+                C2 f;
+                low_fac_global<R>(a.virt, (int)j, gi, lane & 1, f.x, f.y);
+                s_vf[wl][k][j][lane & 1] = f;
+            }
+            if ((lane & 15) == 0 && k < leaf_cnt) {
+                C2 p = reinterpret_cast<const C2 *>(a.virt_in)[afirst + k];
+                low_diag(a.virt, gi, [&](int d, uint32_t idx) { return low_diag_global<R>(a.virt, d, idx); }, p.x, p.y);
+                s_vp[wl][k] = p;
+            }
+            __syncwarp();
+            auto img_w = [&](uint32_t i) -> double {
+                const uint32_t x = i >> a.cond_bits;
+                auto fac = [&](int m, int bit, R &fr, R &fi) {
+                    const C2 f = s_vf[wl][x][m][bit];
+                    fr = f.x; fi = f.y;
+                };
+                const C2 p = s_vp[wl][x];
+                R o_r, o_i;
+                low_image<R, sizeof(R) == 4 ? 2 : 1>(fac, a.cond_bits, p.x, p.y, i & (uint32_t)(nb - 1), o_r, o_i);
+                return (double)o_r * (double)o_r + (double)o_i * (double)o_i;
+            };
+            const uint32_t c = warp_pick(img_w, leaf_cnt * (uint32_t)nb, u, lane);
+            within = (uint64_t)(c >> a.cond_bits) + ((uint64_t)(c & (uint32_t)(nb - 1)) << a.n_active);
+        } else if (a.cond_low) {
             // rotated expansion: the (x, image) pairs of the leaf are one contiguous run, x-major
             const uint32_t c = warp_pick([&](uint32_t i) { return amp_w((afirst << a.cond_bits) + i); },
                                          leaf_cnt * (uint32_t)nb, u, lane);
@@ -2154,9 +2262,12 @@ static __global__ void __launch_bounds__(kThreads) k_released_keys(const __grid_
 // ----------------------------------------------------------------------------------
 // contiguous kept set (QCMRF: the first 2^n amplitudes): probs[i] = |amp_i|^2 and a
 // deterministic two-stage sum (per-block partials, then k_tree_level).
-template <typename R>
+// VIRT: the rotated pass that produced the state was left unwritten; `state` is its input and amplitude i is image 0
+// of input i, computed with the pass's arguments `va` (same loop, same order of the sums).
+template <typename R, bool VIRT>
 __global__ void __launch_bounds__(kThreads) k_probs_prefix(const void *state, uint64_t count, int shift, double *probs, double *partial,
-                                                           uint64_t bstate = 0, uint64_t bprobs = 0, uint64_t bpartial = 0) {
+                                                           uint64_t bstate, uint64_t bprobs, uint64_t bpartial,
+                                                           const __grid_constant__ ExpandTreeArgs va) {
     __shared__ double wsum[kThreads / 32];
     state = batch_ptr(state, bstate);
     if (probs) probs = batch_ptr(probs, bprobs);
@@ -2165,7 +2276,16 @@ __global__ void __launch_bounds__(kThreads) k_probs_prefix(const void *state, ui
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += stride) {
         double w;
-        if constexpr (sizeof(R) == 4) {
+        if constexpr (VIRT) {
+            using C2 = typename CplxOf<R>::T;
+            C2 p = reinterpret_cast<const C2 *>(state)[i];
+            const uint64_t gi = i | va.rank_bits;
+            low_diag(va, gi, [&](int d, uint32_t idx) { return low_diag_global<R>(va, d, idx); }, p.x, p.y);
+            R o_r, o_i;
+            low_image<R, sizeof(R) == 4 ? 2 : 1>([&](int m, int bit, R &fr, R &fi) { low_fac_global<R>(va, m, gi, bit, fr, fi); },
+                                                 va.M, p.x, p.y, 0u, o_r, o_i);
+            w = (double)o_r * (double)o_r + (double)o_i * (double)o_i;
+        } else if constexpr (sizeof(R) == 4) {
             const float2 t = reinterpret_cast<const float2 *>(state)[i << shift];
             w = (double)t.x * (double)t.x + (double)t.y * (double)t.y;
         } else {
