@@ -277,6 +277,52 @@ int qcm_run_batch_small(int device, int precision, int n_circuits,
                         uint64_t shots, uint64_t seed,
                         uint64_t *keys_out, double *probs_out, double *kept_out,
                         double *device_ms_out);
+/* qcm_run_batch_small, then every key's measured clbits flipped by readout errors before the keys are copied out.
+ * readout: [n_circuits][64][2] doubles, per clbit P(read 1 | outcome 0), P(read 0 | outcome 1) (zero for an
+ * unmeasured clbit); NULL: no flips.  Shot s of circuit c draws clbit b's flip from Philox4x32-10 keyed
+ * (seed ^ readout key, stream of c) at counter s * 16 + b / 4 (word b % 4): never a counter of the outcome draw.   */
+int qcm_run_batch_small_readout(int device, int precision, int n_circuits,
+                                const int32_t *n_qubits, const int64_t *op_begin,
+                                const qcm_op *ops, const double *tables, size_t n_tables,
+                                const int32_t *clbit_qubit, const int32_t *n_clbits, const double *readout,
+                                const uint64_t *ps_mask, const uint64_t *ps_value, const int32_t *ps_bits,
+                                const uint64_t *stream_ids, uint64_t shots, uint64_t seed,
+                                uint64_t *keys_out, double *probs_out, double *kept_out, double *device_ms_out);
+
+/* -- noisy shots: Pauli-error trajectories of small circuits --------------------------------------------- */
+/* One unfused gate: `m` (2x2, row-major re/im, fp64) on `target` wherever (index & ctrl_mask) == ctrl_value; then,
+ * when channel >= 0, the Pauli channel channels[channel].                                                        */
+typedef struct {
+    double m[8];
+    int32_t target;
+    uint32_t ctrl_mask;
+    uint32_t ctrl_value;
+    int32_t channel;            /* -1: no error after this gate */
+} qcm_gate;
+
+/* A Pauli channel on 1 or 2 qubits: Pauli k (code (k >> 2j) & 3 on qubit[j]: 0 I, 1 X, 2 Y, 3 Z) has probability
+ * cum[k] - cum[k-1]; cum[n_paulis - 1] == 1.  qubit[1] == -1 for a 1-qubit channel.                              */
+typedef struct {
+    double cum[16];
+    int32_t n_paulis;           /* 4 or 16 */
+    int32_t qubit[2];
+    int32_t pad;
+} qcm_channel;
+
+/* Noisy shots of many circuits in one call, no fusion: every shot of circuit c (n_qubits[c] <=
+ * qcm_small_max_qubits, gates gates[gate_begin[c] .. gate_begin[c+1])) is an independent trajectory from |0..0>:
+ * after gate g the channel draws one Pauli from Philox4x32-10 keyed (seed ^ noise key, stream) at counter
+ * shot * G_c + g (G_c gates in circuit c); the outcome is drawn from |psi|^2 as qcm_run_batch_small draws it; the
+ * key is built from clbit_qubit[64*c ..] and n_clbits[c] as there and flipped by `readout` as in
+ * qcm_run_batch_small_readout (NULL: no readout error).  keys_out is [n_circuits][shots].  Channel indices are
+ * global (into `channels`).  QCM_ERR_UNSUPPORTED above qcm_small_max_qubits qubits; QCM_ERR_INVALID on a
+ * malformed gate, channel or a trajectory whose norm is not finite and positive.  No CPU fallback.              */
+int qcm_run_noisy_small(int device, int precision, int n_circuits, const int32_t *n_qubits,
+                        const int64_t *gate_begin, const qcm_gate *gates,
+                        const qcm_channel *channels, int n_channels,
+                        const int32_t *clbit_qubit, const int32_t *n_clbits, const double *readout,
+                        const uint64_t *stream_ids, uint64_t shots, uint64_t seed,
+                        uint64_t *keys_out, double *device_ms_out);
 
 /* -- batched sweeps ----------------------------------------------------------------- */
 /* A theta / beta sweep over ONE graph (QCMRF's `beta`, /root/reference/QCMRF.py:21,154; BASELINE config 3) is B circuits

@@ -44,7 +44,12 @@ SYMBOLS = ['qcm_abi_version', 'qcm_device_count', 'qcm_last_error', 'qcm_create'
            'qcm_postselect_resident', 'qcm_fetch_probs', 'qcm_sample_batched', 'qcm_sample_released_batched',
            'qcm_sample_sharded_devmass', 'qcm_mrf_exact', 'qcm_mrf_last_error', 'qcm_gather_flag_words',
            'qcm_run_gather_block_inplace', 'qcm_set_deferred', 'qcm_host_alloc', 'qcm_host_free',
-           'qcm_tree_total_device', 'qcm_mark', 'qcm_wait']
+           'qcm_tree_total_device', 'qcm_mark', 'qcm_wait', 'qcm_run_batch_small_readout', 'qcm_run_noisy_small']
+
+#: qcm_gate and qcm_channel of include/qcmrf_b200.h (the noisy-shot launch)
+GATE_DTYPE = np.dtype([('m', '<f8', (8,)), ('target', '<i4'), ('ctrl_mask', '<u4'), ('ctrl_value', '<u4'),
+                       ('channel', '<i4')])
+CHANNEL_DTYPE = np.dtype([('cum', '<f8', (16,)), ('n_paulis', '<i4'), ('qubit', '<i4', (2,)), ('pad', '<i4')])
 
 
 def lib():
@@ -75,6 +80,9 @@ def lib():
     L.qcm_small_max_qubits.argtypes = [i32]
     L.qcm_run_batch_small.argtypes = [i32, i32, i32, vp, vp, vp, vp, ctypes.c_size_t, vp, vp, vp, vp, vp, vp,
                                       u64, u64, vp, vp, vp, ctypes.POINTER(dbl)]
+    L.qcm_run_batch_small_readout.argtypes = [i32, i32, i32, vp, vp, vp, vp, ctypes.c_size_t, vp, vp, vp, vp, vp, vp, vp,
+                                              u64, u64, vp, vp, vp, ctypes.POINTER(dbl)]
+    L.qcm_run_noisy_small.argtypes = [i32, i32, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, u64, u64, vp, ctypes.POINTER(dbl)]
     L.qcm_state_ptr.argtypes = [vp, ctypes.POINTER(vp), ctypes.POINTER(u64)]
     L.qcm_set_active.argtypes = [vp, i32]
     L.qcm_get_active.argtypes = [vp, ctypes.POINTER(i32)]
@@ -111,6 +119,7 @@ def lib():
     if L.qcm_abi_version() != 1:
         raise RuntimeError('qcmrf_b200: ABI version mismatch')
     assert OP_DTYPE.itemsize == 72, OP_DTYPE.itemsize
+    assert GATE_DTYPE.itemsize == 80 and CHANNEL_DTYPE.itemsize == 144
     _lib = L
     return L
 
@@ -408,9 +417,10 @@ def small_max_qubits(precision='double'):
 
 
 def run_batch_small(plans, clbit_maps, ps, shots, seed, precision='double', device=0, want_probs=True,
-                    stream_ids=None):
+                    stream_ids=None, readout=None):
     """plans: list of fusion.Plan (fully materialised); clbit_maps: list of int arrays
-    (clbit -> physical qubit or -1); ps: list of (mask, value, bits).  Returns
+    (clbit -> physical qubit or -1); ps: list of (mask, value, bits); readout: None or (n, 64, 2) per-clbit flip
+    probabilities applied to the keys on the device (qcm_run_batch_small_readout).  Returns
     (keys[n][shots] uint64, probs list, kept array, device_ms)."""
     n = len(plans)
     nq = np.array([p.n_phys for p in plans], dtype=np.int32)
@@ -440,13 +450,57 @@ def run_batch_small(plans, clbit_maps, ps, shots, seed, precision='double', devi
     ms = ctypes.c_double()
     prec = QCM_C64 if precision in ('single', 'c64', 32) else QCM_C128
     sid = None if stream_ids is None else np.ascontiguousarray(stream_ids, dtype=np.uint64)
-    rc = lib().qcm_run_batch_small(int(device), prec, n, _ptr(nq), _ptr(op_begin), _ptr(ops), _ptr(tabs), tabs.size,
-                                   _ptr(cq), _ptr(ncl), _ptr(pm), _ptr(pv), _ptr(pb), _ptr(sid), int(shots), int(seed),
-                                   _ptr(keys), _ptr(probs), _ptr(kept), ctypes.byref(ms))
+    if readout is None:
+        rc = lib().qcm_run_batch_small(int(device), prec, n, _ptr(nq), _ptr(op_begin), _ptr(ops), _ptr(tabs), tabs.size,
+                                       _ptr(cq), _ptr(ncl), _ptr(pm), _ptr(pv), _ptr(pb), _ptr(sid), int(shots), int(seed),
+                                       _ptr(keys), _ptr(probs), _ptr(kept), ctypes.byref(ms))
+    else:
+        ro = np.ascontiguousarray(readout, dtype=np.float64)
+        assert ro.shape == (n, 64, 2), ro.shape
+        rc = lib().qcm_run_batch_small_readout(int(device), prec, n, _ptr(nq), _ptr(op_begin), _ptr(ops), _ptr(tabs),
+                                               tabs.size, _ptr(cq), _ptr(ncl), _ptr(ro), _ptr(pm), _ptr(pv), _ptr(pb),
+                                               _ptr(sid), int(shots), int(seed), _ptr(keys), _ptr(probs), _ptr(kept),
+                                               ctypes.byref(ms))
     if rc:
         raise NativeError(rc, 'qcm_run_batch_small failed')
     plist = [probs[pbeg[i]:pbeg[i + 1]] for i in range(n)] if want_probs else None
     return keys, plist, kept, ms.value
+
+
+def run_noisy_small(encoded, shots, seed, precision='double', device=0, stream_ids=None):
+    """Noisy shots of noise.EncodedNoise programs (qcm_run_noisy_small): one trajectory per shot.  Returns
+    (keys[n][shots] uint64, device_ms)."""
+    n = len(encoded)
+    nq = np.array([e.n_qubits for e in encoded], dtype=np.int32)
+    gate_begin = np.concatenate([[0], np.cumsum([e.n_gates for e in encoded])]).astype(np.int64)
+    gates = np.zeros(int(gate_begin[-1]), dtype=GATE_DTYPE)
+    chans, coff = [], 0
+    for i, e in enumerate(encoded):
+        g = gates[gate_begin[i]:gate_begin[i + 1]]
+        g['m'], g['target'], g['ctrl_mask'], g['ctrl_value'] = e.matrix, e.target, e.ctrl_mask, e.ctrl_value
+        g['channel'] = np.where(e.channel >= 0, e.channel + coff, -1)
+        ch = np.zeros(len(e.n_paulis), dtype=CHANNEL_DTYPE)
+        ch['cum'], ch['n_paulis'], ch['qubit'] = e.cum, e.n_paulis, e.chan_qubits
+        chans.append(ch)
+        coff += len(ch)
+    channels = np.concatenate(chans) if chans else np.zeros(0, dtype=CHANNEL_DTYPE)
+    cq = np.full((n, 64), -1, dtype=np.int32)
+    ncl = np.zeros(n, dtype=np.int32)
+    ro = np.zeros((n, 64, 2))
+    for i, e in enumerate(encoded):
+        cq[i, :e.n_clbits] = e.clbit_map
+        ncl[i] = e.n_clbits
+        ro[i] = e.readout
+    keys = np.empty((n, int(shots)), dtype=np.uint64)
+    sid = None if stream_ids is None else np.ascontiguousarray(stream_ids, dtype=np.uint64)
+    ms = ctypes.c_double()
+    prec = QCM_C64 if precision in ('single', 'c64', 32) else QCM_C128
+    rc = lib().qcm_run_noisy_small(int(device), prec, n, _ptr(nq), _ptr(gate_begin), _ptr(gates), _ptr(channels),
+                                   len(channels), _ptr(cq), _ptr(ncl), _ptr(ro) if ro.any() else None, _ptr(sid),
+                                   int(shots), int(seed), _ptr(keys), ctypes.byref(ms))
+    if rc:
+        raise NativeError(rc, 'qcm_run_noisy_small failed')
+    return keys, ms.value
 
 
 def mrf_exact(cliques, weights, n=None, want_pmf=True, want_energies=False, device=0):

@@ -24,13 +24,14 @@ from typing import List, Optional, Sequence
 
 import numpy as np
 
-from . import _native, fusion, ir, plancache
+from . import _native, fusion, ir, noise, plancache
 
 __all__ = ['B200Simulator', 'Job', 'Result', 'Counts']
 
 _FUSION_MODES = ('off', 'clique', 'blocked')
 #: most sweep points one batched handle holds (the engine's limit: they are the grid's y dimension)
 SWEEP_MAX_POINTS = 65535
+_FROM_OPTIONS = object()
 
 
 class Counts(dict):
@@ -162,11 +163,17 @@ class Result:
             return [e['counts'] for e in self._entries]
         return self._entries[self._idx(experiment)]['counts']
 
+    def _exact(self, experiment):
+        e = self._entries[self._idx(experiment)]
+        if e['meta'].get('noise'):
+            raise ValueError('a noisy experiment has no exact pmf or success probability: its counts are the result')
+        return e
+
     def postselected_probabilities(self, experiment=None):
         """(p, delta): exact pmf over the n variable qubits conditioned on every other
         measured-out qubit being 0 (index: x_0 = MSB, as eval.py:100-101) and the success
-        probability delta."""
-        e = self._entries[self._idx(experiment)]
+        probability delta.  ValueError for an experiment run with noise."""
+        e = self._exact(experiment)
         if e.get('pmf') is not None:                        # normalised while the list's next circuit was running
             return e['pmf'], e['kept']
         if e['probs'] is None:
@@ -178,7 +185,7 @@ class Result:
         return p, kept
 
     def success_probability(self, experiment=None):
-        return self._entries[self._idx(experiment)]['kept']
+        return self._exact(experiment)['kept']
 
     def metadata(self, experiment=None):
         return self._entries[self._idx(experiment)]['meta']
@@ -218,11 +225,11 @@ class B200Simulator:
     options: precision 'double'|'single'; fusion 'off'|'clique'|'blocked';
     block_max 1..5 (targets per blocked pass), expand_max <= 8 (targets of a pass that only
     materialises new qubits); device; seed (None = fresh entropy, as
-    the unseeded Aer run of the reference)."""
+    the unseeded Aer run of the reference); noise_model (a noise.NoiseModel, or None: ideal)."""
 
     def __init__(self, name='qasm_simulator', device=0, precision='double', fusion='blocked', block_max=4,
                  seed=None, small_batch=True, small_fusion='clique', width='full', expand_max=8, plan_cache=True,
-                 sweep_batch=True, sweep_state_bytes=1 << 28, sweep_bytes=32 << 30):
+                 sweep_batch=True, sweep_state_bytes=1 << 28, sweep_bytes=32 << 30, noise_model=None):
         if fusion not in _FUSION_MODES:
             raise ValueError('fusion must be one of %r' % (_FUSION_MODES,))
         if width not in ('full', 'release'):
@@ -253,6 +260,7 @@ class B200Simulator:
         self.sweep_batch = sweep_batch
         self.sweep_state_bytes = int(sweep_state_bytes)
         self.sweep_bytes = int(sweep_bytes)
+        self.noise_model = noise_model
 
     def name(self):
         return self._name
@@ -388,12 +396,14 @@ class B200Simulator:
         return probs, kept
 
     # -- public API ---------------------------------------------------------------------
-    def run(self, circuits, shots=1024, seed=None, precision=None, n_vars=None, stream_ids=None, pmf=None, **options):
+    def run(self, circuits, shots=1024, seed=None, precision=None, n_vars=None, stream_ids=None, pmf=None,
+            noise_model=_FROM_OPTIONS, **options):
         """stream_ids: Philox stream per circuit (default: its index in the list) -- a batch split over
         several GPUs passes the global indices so that the counts do not depend on the partition.
         pmf: sweeps only (circuits of one structure run through one batched handle) -- True copies every point's
         post-selected vector to the host, None (default) leaves them on the GPU until
-        Result.postselected_probabilities(i) asks for one, False computes only delta."""
+        Result.postselected_probabilities(i) asks for one, False computes only delta.
+        noise_model: overrides the simulator's for this call (see _run_noisy)."""
         t0 = time.perf_counter()
         single = not isinstance(circuits, (list, tuple))
         circs = [circuits] if single else list(circuits)
@@ -406,6 +416,11 @@ class B200Simulator:
         small_max = _native.small_max_qubits(precision)
         entries = [None] * len(circs)
         sid = (lambda i: i) if stream_ids is None else (lambda i: int(stream_ids[i]))
+        if noise_model is _FROM_OPTIONS:
+            noise_model = self.noise_model
+        if noise_model is not None and not noise_model.is_ideal():
+            if self._run_noisy(circs, entries, noise_model, shots, seed, precision, n_vars, sid, small_max):
+                return Job(Result(entries, single, self._name, seed, shots, time.perf_counter() - t0))
         small_ids, small_prep = [], []
         large = []
         fast_sweeps = []                                      # (indices, prepared sweep): same-graph QCMRF lists at release width
@@ -500,16 +515,65 @@ class B200Simulator:
                 [pr.plan for pr in small_prep], [pr.clbit_map for pr in small_prep], ps, shots, seed,
                 precision=precision, device=self.device, want_probs=True, stream_ids=[sid(i) for i in small_ids])
             for j, (i, pr) in enumerate(zip(small_ids, small_prep)):
-                has_ps = pr.ps is not None
-                entries[i] = {
-                    'circuit': circs[i], 'name': pr.name,
-                    'counts': _keys_to_counts(keys[j], pr.prog.n_clbits) if shots else None,
-                    'probs': probs[j].copy() if has_ps else None, 'kept': float(kept[j]) if has_ps else None,
-                    'meta': {'path': 'batch_small', 'n_qubits': pr.prog.n_qubits, 'n_phys': pr.plan.n_phys,
-                             'passes': pr.plan.n_passes, 'gates_in': pr.fc.n_gates_in, 'batch_device_ms': ms,
-                             'philox_stream': sid(i)}}
+                entries[i] = self._small_entry(circs[i], pr, keys[j] if shots else None, probs[j], kept[j], ms, sid(i))
         res = Result(entries, single, self._name, seed, shots, time.perf_counter() - t0)
         return Job(res)
+
+    @staticmethod
+    def _small_entry(circ, pr, keys, probs, kept, ms, stream):
+        has_ps = pr.ps is not None
+        return {'circuit': circ, 'name': pr.name,
+                'counts': _keys_to_counts(keys, pr.prog.n_clbits) if keys is not None else None,
+                'probs': probs.copy() if has_ps else None, 'kept': float(kept) if has_ps else None,
+                'meta': {'path': 'batch_small', 'n_qubits': pr.prog.n_qubits, 'n_phys': pr.plan.n_phys,
+                         'passes': pr.plan.n_passes, 'gates_in': pr.fc.n_gates_in, 'batch_device_ms': ms,
+                         'philox_stream': stream}}
+
+    def _run_noisy(self, circs, entries, model, shots, seed, precision, n_vars, sid, small_max):
+        """Fill `entries` for a call under a noise model; False (nothing filled) when no error of the model applies
+        to any circuit, which then runs exactly as without a model.  A circuit is noisy when an error with a
+        non-identity probability above 0 follows one of its gates or reads one of its measured qubits.  A noisy call
+        runs every circuit on the small-circuit path (no sweeps, no release width; ValueError above small_max
+        qubits): circuits with gate errors as one trajectory per shot (qcm_run_noisy_small), the others through the
+        ideal batched kernel, their keys flipped by their readout errors on the device.  Noisy experiments have
+        counts and no exact pmf or success probability."""
+        progs = [ir.lower(c) for c in circs]
+        if any(p.n_clbits > 64 for p in progs):
+            raise ValueError('at most 64 classical bits are supported')
+        enc = [noise.encode(p, model) for p in progs]
+        if not any(e.noisy for e in enc):
+            return False
+        big = [i for i, p in enumerate(progs) if p.n_qubits > small_max]
+        if big:
+            raise ValueError('noisy shots need circuits of at most %d qubits (circuit %d has %d)'
+                             % (small_max, big[0], progs[big[0]].n_qubits))
+        traj = [i for i, e in enumerate(enc) if e.gate_noisy]
+        if traj:
+            keys, ms = _native.run_noisy_small([enc[i] for i in traj], shots, seed, precision=precision,
+                                               device=self.device, stream_ids=[sid(i) for i in traj])
+            for j, i in enumerate(traj):
+                p = progs[i]
+                entries[i] = {'circuit': circs[i], 'name': p.name,
+                              'counts': _keys_to_counts(keys[j], p.n_clbits) if shots else None, 'probs': None,
+                              'kept': None,
+                              'meta': {'path': 'noisy_trajectories', 'noise': True, 'n_qubits': p.n_qubits,
+                                       'gates': enc[i].n_gates, 'channels': len(enc[i].n_paulis),
+                                       'noisy_device_ms': ms, 'philox_stream': sid(i)}}
+        rest = [i for i, e in enumerate(enc) if not e.gate_noisy]
+        if rest:
+            prep = [self.prepare(progs[i], n_vars=n_vars, small=True) for i in rest]
+            ps = [pr.ps if pr.ps is not None else (0, 0, 0) for pr in prep]
+            readout = np.stack([enc[i].readout for i in rest]) if any(enc[i].readout_noisy for i in rest) else None
+            keys, probs, kept, ms = _native.run_batch_small(
+                [pr.plan for pr in prep], [pr.clbit_map for pr in prep], ps, shots, seed, precision=precision,
+                device=self.device, want_probs=True, stream_ids=[sid(i) for i in rest], readout=readout)
+            for j, (i, pr) in enumerate(zip(rest, prep)):
+                e = self._small_entry(circs[i], pr, keys[j] if shots else None, probs[j], kept[j], ms, sid(i))
+                if enc[i].noisy:
+                    e['probs'] = e['kept'] = None
+                    e['meta']['noise'] = True
+                entries[i] = e
+        return True
 
     # -- sweeps: circuits of one structure through a batched handle ------------------------------------
     def _sweep_signature(self, pr, precision):

@@ -11,8 +11,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libqcmrf_b200.so')
-SOURCES = ['qcm_api.cu', 'qcm_small.cu', 'qcm_mrf.cu']
-HEADERS = [os.path.join(CSRC, 'qcm_kernels.cuh'), os.path.join(ROOT, 'include', 'qcmrf_b200.h')]
+SOURCES = ['qcm_api.cu', 'qcm_small.cu', 'qcm_mrf.cu', 'qcm_noise.cu']
+HEADERS = [os.path.join(CSRC, 'qcm_kernels.cuh'), os.path.join(CSRC, 'qcm_noise.h'), os.path.join(ROOT, 'include', 'qcmrf_b200.h')]
 
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC',

@@ -13,13 +13,12 @@
 #include <vector>
 
 #include "qcm_kernels.cuh"
+#include "qcm_noise.h"
 #include "qcmrf_b200.h"
 
 using namespace qcm;
 
 namespace {
-
-constexpr int kSmallMaxQubits = 13;
 
 struct SmallArgs {
     int n_circuits;
@@ -190,22 +189,11 @@ __global__ void __launch_bounds__(kThreads) k_small(const SmallArgs a) {
 
 thread_local std::string g_small_error;
 
-// Per-device, grow-only work space of the batched path: ONE device buffer, ONE pinned host buffer for the
-// inputs (a single H2D copy), one stream and two events -- created once, reused by every call (the first
-// version paid ~15 cudaMalloc + cudaFree per batch, 10-25 ms next to a 0.07 ms kernel).  Guarded by a mutex:
-// calls on the same device serialise.
-struct SmallArena {
-    std::mutex mu;
-    void *dev = nullptr;
-    size_t dev_cap = 0;
-    void *pin = nullptr;
-    size_t pin_cap = 0;
-    cudaStream_t st = nullptr;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-};
-SmallArena g_arena[64];
+}  // namespace
 
-inline size_t up256(size_t x) { return (x + 255) & ~size_t(255); }
+namespace qcm {
+
+SmallArena g_arena[64];
 
 cudaError_t arena_reserve(SmallArena &A, size_t dev_bytes, size_t pin_bytes) {
     cudaError_t e;
@@ -229,21 +217,16 @@ cudaError_t arena_reserve(SmallArena &A, size_t dev_bytes, size_t pin_bytes) {
     return cudaSuccess;
 }
 
-}  // namespace
+}  // namespace qcm
 
+namespace {
 
-
-extern "C" {
-
-int qcm_small_max_qubits(int precision) {
-    return (precision == QCM_C64 || precision == QCM_C128) ? kSmallMaxQubits : 0;
-}
-
-int qcm_run_batch_small(int device, int precision, int n_circuits, const int32_t *n_qubits, const int64_t *op_begin,
-                        const qcm_op *ops, const double *tables, size_t n_tables, const int32_t *clbit_qubit,
-                        const int32_t *n_clbits, const uint64_t *ps_mask, const uint64_t *ps_value, const int32_t *ps_bits,
-                        const uint64_t *stream_ids, uint64_t shots, uint64_t seed, uint64_t *keys_out, double *probs_out, double *kept_out,
-                        double *device_ms_out) {
+// qcm_run_batch_small; with `readout` (qcm_run_batch_small_readout) the keys are flipped on the device before the copy.
+int run_batch_small(int device, int precision, int n_circuits, const int32_t *n_qubits, const int64_t *op_begin,
+                    const qcm_op *ops, const double *tables, size_t n_tables, const int32_t *clbit_qubit,
+                    const int32_t *n_clbits, const double *readout, const uint64_t *ps_mask, const uint64_t *ps_value,
+                    const int32_t *ps_bits, const uint64_t *stream_ids, uint64_t shots, uint64_t seed, uint64_t *keys_out,
+                    double *probs_out, double *kept_out, double *device_ms_out) {
     if (n_circuits <= 0 || !n_qubits || !op_begin || !ops || !ps_mask || !ps_value || !ps_bits || !kept_out) return QCM_ERR_INVALID;
     if (precision != QCM_C64 && precision != QCM_C128) return QCM_ERR_INVALID;
     if (shots && (!keys_out || !clbit_qubit || !n_clbits)) return QCM_ERR_INVALID;
@@ -290,6 +273,7 @@ int qcm_run_batch_small(int device, int precision, int n_circuits, const int32_t
                  o_tab = take(n_tables * 8), o_pm = take(nc * 8), o_pv = take(nc * 8), o_psb = take(nc * 4),
                  o_pb = take((nc + 1) * 8), o_sid = take(stream_ids ? nc * 8 : 0), o_cq = take(shots ? 64 * nc * 4 : 0),
                  o_ncl = take(shots ? nc * 4 : 0);
+    const size_t o_ro = (shots && readout) ? take(nc * 128 * 8) : 0;
     const size_t in_bytes = off;
     const size_t o_keys = take(shots ? shots * nc * 8 : 0), o_kept = take(nc * 8), o_status = take(nc * 4),
                  o_probs = take(probs_out ? (size_t)pbeg[n_circuits] * 8 : 0);
@@ -311,6 +295,7 @@ int qcm_run_batch_small(int device, int precision, int n_circuits, const int32_t
     if (shots) {
         memcpy(hp + o_cq, clbit_qubit, 64 * nc * 4);
         memcpy(hp + o_ncl, n_clbits, nc * 4);
+        if (readout) memcpy(hp + o_ro, readout, nc * 128 * 8);
     }
     SM_CUDA(cudaMemcpyAsync(dp, hp, in_bytes, cudaMemcpyHostToDevice, A.st));
     if (probs_out) SM_CUDA(cudaMemsetAsync(dp + o_probs, 0, (size_t)pbeg[n_circuits] * 8, A.st));
@@ -342,6 +327,9 @@ int qcm_run_batch_small(int device, int precision, int n_circuits, const int32_t
         k_small<double><<<n_circuits, kThreads, smem, A.st>>>(a);
     }
     SM_CUDA(cudaGetLastError());
+    if (shots && readout)
+        SM_CUDA(launch_readout_keys(A.st, n_circuits, shots, seed, a.stream_ids, a.n_clbits, (const double *)(dp + o_ro),
+                                    a.keys_out));
     SM_CUDA(cudaEventRecord(A.e1, A.st));
     SM_CUDA(cudaMemcpyAsync(kept_out, dp + o_kept, nc * sizeof(double), cudaMemcpyDeviceToHost, A.st));
     SM_CUDA(cudaMemcpyAsync(status.data(), dp + o_status, nc * sizeof(int32_t), cudaMemcpyDeviceToHost, A.st));
@@ -358,6 +346,35 @@ int qcm_run_batch_small(int device, int precision, int n_circuits, const int32_t
 done:
     return rc;
 #undef SM_CUDA
+}
+
+}  // namespace
+
+extern "C" {
+
+int qcm_small_max_qubits(int precision) {
+    return (precision == QCM_C64 || precision == QCM_C128) ? kSmallMaxQubits : 0;
+}
+
+int qcm_run_batch_small(int device, int precision, int n_circuits, const int32_t *n_qubits, const int64_t *op_begin,
+                        const qcm_op *ops, const double *tables, size_t n_tables, const int32_t *clbit_qubit,
+                        const int32_t *n_clbits, const uint64_t *ps_mask, const uint64_t *ps_value, const int32_t *ps_bits,
+                        const uint64_t *stream_ids, uint64_t shots, uint64_t seed, uint64_t *keys_out, double *probs_out, double *kept_out,
+                        double *device_ms_out) {
+    return run_batch_small(device, precision, n_circuits, n_qubits, op_begin, ops, tables, n_tables, clbit_qubit, n_clbits,
+                           nullptr, ps_mask, ps_value, ps_bits, stream_ids, shots, seed, keys_out, probs_out, kept_out,
+                           device_ms_out);
+}
+
+int qcm_run_batch_small_readout(int device, int precision, int n_circuits, const int32_t *n_qubits, const int64_t *op_begin,
+                                const qcm_op *ops, const double *tables, size_t n_tables, const int32_t *clbit_qubit,
+                                const int32_t *n_clbits, const double *readout, const uint64_t *ps_mask,
+                                const uint64_t *ps_value, const int32_t *ps_bits, const uint64_t *stream_ids, uint64_t shots,
+                                uint64_t seed, uint64_t *keys_out, double *probs_out, double *kept_out,
+                                double *device_ms_out) {
+    return run_batch_small(device, precision, n_circuits, n_qubits, op_begin, ops, tables, n_tables, clbit_qubit, n_clbits,
+                           readout, ps_mask, ps_value, ps_bits, stream_ids, shots, seed, keys_out, probs_out, kept_out,
+                           device_ms_out);
 }
 
 }  // extern "C"
