@@ -386,6 +386,15 @@ const char *qcm_mrf_last_error(void);
  * top `g` local qubits, which the caller moves with NCCL (torch.distributed).  These
  * two report the device pointer and byte size so the caller can wrap the state.     */
 int qcm_state_ptr(qcm_handle h, void **dev_ptr_out, uint64_t *bytes_out);
+/* Read-only view of the sampler's sum tree (for tests and diagnostics): the device pointer and
+ * entry count (doubles) of level `level`, 0 = the chunk sums over 2^10 amplitudes ... top, and
+ * -1 = the finer level under level 0 when the tree has one.  *n_levels_out (optional) receives
+ * the number of levels above the amplitudes.  The finer level of an unwritten last pass is not
+ * stored (the sampler computes the entries it reads): -1 then writes it, with the sampler's
+ * arithmetic, into a handle buffer and synchronises the handle's stream.  Nothing else is built or
+ * written: QCM_ERR_INVALID when the handle holds no valid tree or the level does not exist.
+ * Batched handles: point 0.                                                                   */
+int qcm_tree_level(qcm_handle h, int level, const double **dev_ptr_out, uint64_t *n_out, int *n_levels_out);
 int qcm_set_active(qcm_handle h, int n_active);
 int qcm_get_active(qcm_handle h, int *n_active_out);
 

@@ -44,7 +44,7 @@ SYMBOLS = ['qcm_abi_version', 'qcm_device_count', 'qcm_last_error', 'qcm_create'
            'qcm_postselect_resident', 'qcm_fetch_probs', 'qcm_sample_batched', 'qcm_sample_released_batched',
            'qcm_sample_sharded_devmass', 'qcm_mrf_exact', 'qcm_mrf_last_error', 'qcm_gather_flag_words',
            'qcm_run_gather_block_inplace', 'qcm_set_deferred', 'qcm_host_alloc', 'qcm_host_free',
-           'qcm_tree_total_device', 'qcm_mark', 'qcm_wait', 'qcm_run_batch_small_readout', 'qcm_run_noisy_small']
+           'qcm_tree_total_device', 'qcm_mark', 'qcm_wait', 'qcm_run_batch_small_readout', 'qcm_run_noisy_small', 'qcm_tree_level']
 
 #: qcm_gate and qcm_channel of include/qcmrf_b200.h (the noisy-shot launch)
 GATE_DTYPE = np.dtype([('m', '<f8', (8,)), ('target', '<i4'), ('ctrl_mask', '<u4'), ('ctrl_value', '<u4'),
@@ -84,6 +84,7 @@ def lib():
                                               u64, u64, vp, vp, vp, ctypes.POINTER(dbl)]
     L.qcm_run_noisy_small.argtypes = [i32, i32, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, u64, u64, vp, ctypes.POINTER(dbl)]
     L.qcm_state_ptr.argtypes = [vp, ctypes.POINTER(vp), ctypes.POINTER(u64)]
+    L.qcm_tree_level.argtypes = [vp, i32, ctypes.POINTER(vp), ctypes.POINTER(u64), ctypes.POINTER(i32)]
     L.qcm_set_active.argtypes = [vp, i32]
     L.qcm_get_active.argtypes = [vp, ctypes.POINTER(i32)]
     L.qcm_get_timing.argtypes = [vp, ctypes.POINTER(QcmTiming)]
@@ -387,6 +388,13 @@ class Handle:
         p, b = ctypes.c_void_p(), ctypes.c_uint64()
         self._check(lib().qcm_state_ptr(self._h, ctypes.byref(p), ctypes.byref(b)))
         return p.value, b.value
+
+    def tree_level(self, level):
+        """(device pointer, entry count, number of levels) of one level of the sampler's sum tree, read-only: 0 = the
+        chunk sums ... top, -1 = the finer level under level 0.  Builds nothing; raises when there is no such level."""
+        p, n, nl = ctypes.c_void_p(), ctypes.c_uint64(), ctypes.c_int()
+        self._check(lib().qcm_tree_level(self._h, int(level), ctypes.byref(p), ctypes.byref(n), ctypes.byref(nl)))
+        return p.value, n.value, nl.value
 
     def synchronize(self):
         self._check(lib().qcm_synchronize(self._h))

@@ -80,6 +80,7 @@ struct qcm_sim_s {
     int tree_cond_bits = 0;         // expansion qubits materialised after the tree was built
     int tree_sub_bits = 0;          // subtree holds sums over 2^tree_sub_bits amplitudes ...
     bool tree_has_sub = false;      // ... when this is set (fused checkpoint only)
+    bool tree_sub_input = false;    // ... not stored: the sampler computes it from the input in `scratch` (virtual pass)
     bool tree_sub_strided = false;  // generic tree build: subtree holds k_chunk_sums' 32 lane partials per chunk
     uint64_t n_expand = 0, n_checkpoint = 0;
     double local_mass = 0.0;
@@ -483,13 +484,12 @@ int raise_smem_limit(qcm_handle h, const void *kern) {
     return QCM_OK;
 }
 
-// EMIT = false: the sums-only launch of a virtual last pass (no tables, no stores of the state)
-template <typename R, int V, int MH, int TB, int NW, bool EMIT>
+template <typename R, int V, int MH, int TB, int NW>
 static int launch_low_tb(qcm_handle h, int n_in, BlockPlan &bp) {
-    auto kern = k_expand_low<R, V, MH, TB, NW, EMIT>;
+    auto kern = k_expand_low<R, V, MH, TB, NW>;
     constexpr int warps = NW;
-    size_t smem = EMIT ? low_warp_bytes<R, MH>() * warps + bp.tree_smem : 0;
-    if (EMIT) {
+    size_t smem = low_warp_bytes<R, MH>() * warps + bp.tree_smem;
+    {
         // default: 24 resident warps per SM for complex64 (q34 last pass, profiles/r02_low_ctas_sweep.txt: 8x8 at 5 / 4 / 3 /
         // 2 CTAs per SM 9.72 / 9.67 / 9.65 / 10.02 ms, 4x7 at 10 / 8 / 6 / 5 / 4: 9.78 / 9.72 / 9.66 / 9.74 / 10.00);
         // complex128 CTAs (4 warps, twice the shared memory) already sit at 6 per SM
@@ -509,12 +509,7 @@ static int launch_low_tb(qcm_handle h, int n_in, BlockPlan &bp) {
         args.tree_out = (double *)h->lowpart.p;
     }
     kern<<<1u << (n_in - TB), NW * 32, smem, h->stream>>>(args, h->scratch.p);
-    {
-        char nm[96];
-        if (EMIT) snprintf(nm, sizeof nm, "k_expand_low<%s,%d,MH=%d,TB=%d,NW=%d>", sizeof(R) == 4 ? "float" : "double", V, MH, TB, NW);
-        else snprintf(nm, sizeof nm, "k_expand_low_sums<%s,%d,TB=%d,NW=%d>", sizeof(R) == 4 ? "float" : "double", V, TB, NW);
-        h->cur_kernel = nm;
-    }
+    name_kernel(h, "k_expand_low<%s,%d,MH=%d,TB=%d,NW=%d>", sizeof(R) == 4 ? "float" : "double", V, MH, TB, NW);
     QCM_CUDA(h, cudaGetLastError());
     if (level0) {
         int wbits = 0;
@@ -527,16 +522,42 @@ static int launch_low_tb(qcm_handle h, int n_in, BlockPlan &bp) {
     return QCM_OK;
 }
 
-template <typename R, int V, int MH, bool EMIT = true>
+// the shape of the materialising launch (QCM_LOW_SHAPE), as NW * 100 + TB; complex128 CTAs have always been 4 warps
+// (twice the shared memory per warp)
+template <typename R>
+static int low_shape_for() {
+    return (sizeof(R) == 8 && low_shape() == 808) ? 407 : low_shape();
+}
+
+template <typename R, int V, int MH>
 static int launch_low(qcm_handle h, int n_in, BlockPlan &bp) {
-    // complex128 CTAs have always been 4 warps (twice the shared memory per warp)
-    const int shape = (sizeof(R) == 8 && low_shape() == 808) ? 407 : low_shape();
-    switch (shape) {
-        case 810: return launch_low_tb<R, V, MH, 10, 8, EMIT>(h, n_in, bp);
-        case 407: return launch_low_tb<R, V, MH, 7, 4, EMIT>(h, n_in, bp);
-        case 206: return launch_low_tb<R, V, MH, 6, 2, EMIT>(h, n_in, bp);
-        case 105: return launch_low_tb<R, V, MH, 5, 1, EMIT>(h, n_in, bp);
-        default: return launch_low_tb<R, V, MH, 8, 8, EMIT>(h, n_in, bp);
+    switch (low_shape_for<R>()) {
+        case 810: return launch_low_tb<R, V, MH, 10, 8>(h, n_in, bp);
+        case 407: return launch_low_tb<R, V, MH, 7, 4>(h, n_in, bp);
+        case 206: return launch_low_tb<R, V, MH, 6, 2>(h, n_in, bp);
+        case 105: return launch_low_tb<R, V, MH, 5, 1>(h, n_in, bp);
+        default: return launch_low_tb<R, V, MH, 8, 8>(h, n_in, bp);
+    }
+}
+
+// the sums-only launch of a virtual last pass: level 0, with the association of the materialising launch's shape
+// (k_expand_low_sums)
+template <typename R, int TB, int NW>
+static int launch_low_sums_tb(qcm_handle h, int n_in, const BlockPlan &bp) {
+    const uint64_t chunks = 1ull << (n_in - kChunkBits);
+    k_expand_low_sums<R, TB, NW><<<(unsigned)chunks, kSumsThreads, 0, h->stream>>>(h->scratch.p, bp.trargs.tree_out);
+    name_kernel(h, "k_expand_low_sums<%s,%d,TB=%d,NW=%d>", sizeof(R) == 4 ? "float" : "double", sizeof(R) == 4 ? 2 : 1, TB, NW);
+    return QCM_OK;
+}
+
+template <typename R>
+static int launch_low_sums(qcm_handle h, int n_in, const BlockPlan &bp) {
+    switch (low_shape_for<R>()) {
+        case 810: return launch_low_sums_tb<R, 10, 8>(h, n_in, bp);
+        case 407: return launch_low_sums_tb<R, 7, 4>(h, n_in, bp);
+        case 206: return launch_low_sums_tb<R, 6, 2>(h, n_in, bp);
+        case 105: return launch_low_sums_tb<R, 5, 1>(h, n_in, bp);
+        default: return launch_low_sums_tb<R, 8, 8>(h, n_in, bp);
     }
 }
 
@@ -653,11 +674,11 @@ int launch_block_plan(qcm_handle h, BlockPlan &bp) {
             h->timing.bytes_read += in_bytes;      // the scratch copy: one more read and write of the input
             h->timing.bytes_written += in_bytes;
         }
-        // a virtual pass runs the checkpoint sums only, in the materialising launch's shape (the same level-0
-        // association), and nothing at all without the checkpoint
+        // a virtual pass runs the checkpoint sums only, with the materialising launch's association (the same tree), and
+        // nothing at all without the checkpoint
         const bool launch = !bp.virt || bp.trargs.tree_out;
         if (!launch) rc = QCM_OK;
-        else if (bp.virt) rc = h->prec == QCM_C64 ? launch_low<float, 2, 0, false>(h, n_in, bp) : launch_low<double, 1, 0, false>(h, n_in, bp);
+        else if (bp.virt) rc = h->prec == QCM_C64 ? launch_low_sums<float>(h, n_in, bp) : launch_low_sums<double>(h, n_in, bp);
         else if (h->prec == QCM_C64) rc = launch_low_mh<float, 2>(h, M - 6, n_in, bp);
         else rc = launch_low_mh<double, 1>(h, M - 5, n_in, bp);
         if (rc) return rc;
@@ -671,9 +692,9 @@ int launch_block_plan(qcm_handle h, BlockPlan &bp) {
             h->virt_args = bp.trargs;
             h->virt_args.tree_out = nullptr;     // materialise_last: the tree exists already
             h->virt_smem = bp.tree_smem;
-            if (launch) {                        // algorithmic traffic: the input read, the finer sum level written
+            if (launch) {                        // algorithmic traffic: the input read, level 0 written
                 h->timing.bytes_read += in_bytes;
-                h->timing.bytes_written += sizeof(double) << (n_in - (h->prec == QCM_C64 ? 1 : 0));
+                h->timing.bytes_written += sizeof(double) << (n_in - kChunkBits);
             }
             return QCM_OK;
         }
@@ -1104,6 +1125,7 @@ int tree_finish(qcm_handle h, int na) {
         h->tree_cond_bits = 0;
         h->tree_sub_bits = 0;
         h->tree_has_sub = false;
+        h->tree_sub_input = false;
         return QCM_OK;
     }
     if (h->deferred) {
@@ -1124,6 +1146,7 @@ int tree_finish(qcm_handle h, int na) {
     h->tree_cond_bits = 0;
     h->tree_sub_bits = 0;
     h->tree_has_sub = false;
+    h->tree_sub_input = false;
     return QCM_OK;
 }
 
@@ -1460,6 +1483,40 @@ int qcm_state_ptr(qcm_handle h, void **dev_ptr_out, uint64_t *bytes_out) {
     return QCM_OK;
 }
 
+int qcm_tree_level(qcm_handle h, int level, const double **dev_ptr_out, uint64_t *n_out, int *n_levels_out) {
+    if (!h) return fail(nullptr, QCM_ERR_INVALID, "handle is NULL");
+    if (!h->tree_valid) return fail(h, QCM_ERR_INVALID, "no sum tree");
+    if (level < -1 || level >= h->tree_levels) return fail(h, QCM_ERR_INVALID, "tree level %d of %d", level, h->tree_levels);
+    const double *p;
+    uint64_t n;
+    if (level >= 0) {
+        p = h->tree_ptr[level];
+        n = h->tree_n[level];
+    } else if (h->tree_sub_input) {                // not stored: computed here with the sampler's arithmetic
+        n = 1ull << (h->tree_base_bits - h->tree_sub_bits);
+        int rc = ensure(h, h->subtree, sizeof(double) * n);
+        if (rc) return rc;
+        const unsigned blocks = (unsigned)((n + kThreads - 1) / kThreads);
+        if (h->prec == QCM_C64) k_low_sub_entries<float><<<blocks, kThreads, 0, h->stream>>>(h->scratch.p, n, (double *)h->subtree.p);
+        else k_low_sub_entries<double><<<blocks, kThreads, 0, h->stream>>>(h->scratch.p, n, (double *)h->subtree.p);
+        QCM_CUDA(h, cudaGetLastError());
+        QCM_CUDA(h, cudaStreamSynchronize(h->stream));
+        p = (const double *)h->subtree.p;
+    } else if (h->tree_has_sub) {                  // the fused checkpoint's level: sums over 2^tree_sub_bits amplitudes
+        p = (const double *)h->subtree.p;
+        n = 1ull << (h->tree_base_bits - h->tree_sub_bits);
+    } else if (h->tree_sub_strided) {              // k_chunk_sums' 32 lane partials per chunk
+        p = (const double *)h->subtree.p;
+        n = h->tree_n[0] * 32;
+    } else {
+        return fail(h, QCM_ERR_INVALID, "the tree has no finer level");
+    }
+    if (dev_ptr_out) *dev_ptr_out = p;
+    if (n_out) *n_out = n;
+    if (n_levels_out) *n_levels_out = h->tree_levels;
+    return QCM_OK;
+}
+
 int qcm_set_deferred(qcm_handle h, int deferred) {
     if (!h) return fail(nullptr, QCM_ERR_INVALID, "handle is NULL");
     h->deferred = deferred != 0;
@@ -1675,9 +1732,11 @@ int qcm_run_program(qcm_handle h, const qcm_op *ops, int n_ops, const double *ta
                     const int vbits = (h->prec == QCM_C64) ? 1 : 0;
                     sub_bits = bp.tree ? vbits : vbits + 5;
                     if ((rc = tree_layout(h, op.n_active_in))) return rc;
-                    if ((rc = ensure(h, h->subtree, sizeof(double) << (op.n_active_in - sub_bits)))) return rc;
+                    // a virtual pass stores no finer level: its input stays in `scratch` as long as the tree is valid
+                    // (only a next program writes there), and the sampler computes the entries it reads from it
+                    if (!bp.virt && (rc = ensure(h, h->subtree, sizeof(double) << (op.n_active_in - sub_bits)))) return rc;
                     bp.eargs.tree_out = bp.trargs.tree_out = h->tree_ptr[0];
-                    bp.eargs.sub_out = bp.trargs.sub_out = (double *)h->subtree.p;
+                    bp.eargs.sub_out = bp.trargs.sub_out = bp.virt ? nullptr : (double *)h->subtree.p;
                 }
                 if ((rc = launch_block_plan(h, bp))) return rc;
                 if (checkpoint) {
@@ -1687,6 +1746,7 @@ int qcm_run_program(qcm_handle h, const qcm_op *ops, int n_ops, const double *ta
                     h->tree_cond_low = bp.rotate;
                     h->tree_sub_bits = sub_bits;
                     h->tree_has_sub = true;
+                    h->tree_sub_input = bp.virt;
                     h->tree_for_active = op.n_active_out;
                     h->n_checkpoint++;
                     keep_tree = true;
@@ -2070,7 +2130,8 @@ static int sample_sharded_impl(qcm_handle h, uint64_t shots, uint64_t seed, uint
         a.virt_in = h->scratch.p;
         a.virt = h->virt_args;
     }
-    a.sub = (h->tree_has_sub || h->tree_sub_strided) ? (const double *)h->subtree.p : nullptr;
+    a.sub = ((h->tree_has_sub && !h->tree_sub_input) || h->tree_sub_strided) ? (const double *)h->subtree.p : nullptr;
+    a.sub_in = h->tree_sub_input ? h->scratch.p : nullptr;
     a.sub_bits = h->tree_sub_bits;
     a.sub_strided = (h->tree_sub_strided && !h->tree_has_sub) ? 1 : 0;
     a.bsub = (sizeof(double) * 32) << (h->tree_base_bits - std::min(h->tree_base_bits, kChunkBits));

@@ -1307,6 +1307,22 @@ __device__ __forceinline__ void low_cmul(double ar, double ai, double br, double
     cr = __fma_rn(ar, br, -t);
     ci = __fma_rn(ar, bi, u);
 }
+// |in[x]|^2 in double, the sampler's weight of one input: k_expand_low's checkpoint sums and k_expand_low_sums share
+// it, rounded as nvcc contracted it before (y*y first, then one fma), so both build the same tree.  In complex64 the
+// products are exact and any contraction agrees; in complex128 it is this one.
+__device__ __forceinline__ double low_weight(float x, float y) {
+    return __fma_rn((double)x, (double)x, __dmul_rn((double)y, (double)y));
+}
+__device__ __forceinline__ double low_weight(double x, double y) { return __fma_rn(x, x, __dmul_rn(y, y)); }
+// entry p of the finer sum level of a rotated pass's checkpoint, from the pass's input: complex64 w(2p) + w(2p + 1)
+// (the input pair, even input first), complex128 w(p) -- what k_expand_low stores as its sub_out
+template <typename R>
+__device__ __forceinline__ double low_sub_entry(const void *in, uint64_t p) {
+    using C2 = typename CplxOf<R>::T;
+    const C2 *a = reinterpret_cast<const C2 *>(in);
+    if constexpr (sizeof(R) == 4) return low_weight(a[2 * p].x, a[2 * p].y) + low_weight(a[2 * p + 1].x, a[2 * p + 1].y);
+    else return low_weight(a[p].x, a[p].y);
+}
 // table index of member m at global index gi
 __device__ __forceinline__ uint32_t low_index(const TreeMember &m, uint64_t gi) {
     uint32_t idx = 0;
@@ -1403,9 +1419,7 @@ static __global__ void __launch_bounds__(kThreads) k_group_sum(const double *in,
 // NW: warps per CTA.  The size of the region a CTA writes decides how compact the window of concurrently written addresses
 // is (tools/membench4.cu, profiles/r02_notes.md: a bare sequential writer loses 5 % going from 32 KiB to 512 KiB per CTA),
 // so small CTAs -- few warps, one batch of 32 inputs each -- are the default shape.
-// EMIT = false: the sums only (input load, sub_out, level 0) -- the result is left unwritten and its readers compute the
-// images they need (the virtual last pass, DESIGN.md 3); same TB / NW as the materialising launch, so the same tree.
-template <typename R, int V, int MH, int TB, int NW = low_threads<R>() / 32, bool EMIT = true>
+template <typename R, int V, int MH, int TB, int NW = low_threads<R>() / 32>
 __global__ void __launch_bounds__(NW * 32) k_expand_low(const __grid_constant__ ExpandTreeArgs a, const void *__restrict__ in) {
     constexpr int LB = V == 2 ? 6 : 5;                   // image bits covered by one warp store
     constexpr int J0 = V == 2 ? 1 : 0;                   // first lane-indexed member (member 0 is the vector slot for V == 2)
@@ -1430,21 +1444,19 @@ __global__ void __launch_bounds__(NW * 32) k_expand_low(const __grid_constant__ 
     };
     // the first input amplitude is requested before anything else (its DRAM latency then overlaps the table staging)
     C2 next_in = in_at(x_first(0), 2 * kWarps);
-    if constexpr (EMIT) {
-        for (int j = 0; j < M; ++j) {                     // column 0 of every 2x2: (m00, m10)
-            const int n = 1 << a.mem[j].n_ctrl;
-            for (int i = threadIdx.x; i < n; i += blockDim.x) {
-                const R *src = gt + a.mem[j].src_off + 8 * i;
-                R *dst = tab + a.mem[j].tab_off + 4 * i;
-                dst[0] = src[0]; dst[1] = src[1]; dst[2] = src[4]; dst[3] = src[5];
-            }
+    for (int j = 0; j < M; ++j) {                         // column 0 of every 2x2: (m00, m10)
+        const int n = 1 << a.mem[j].n_ctrl;
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            const R *src = gt + a.mem[j].src_off + 8 * i;
+            R *dst = tab + a.mem[j].tab_off + 4 * i;
+            dst[0] = src[0]; dst[1] = src[1]; dst[2] = src[4]; dst[3] = src[5];
         }
-        for (int d = 0; d < a.n_diag; ++d) {
-            const int n = 2 << a.diag[d].n_ctrl;
-            for (int i = threadIdx.x; i < n; i += blockDim.x) tab[a.diag[d].tab_off + i] = gt[a.diag[d].src_off + i];
-        }
-        __syncthreads();                                  // the only block-level barrier: member tables staged
     }
+    for (int d = 0; d < a.n_diag; ++d) {
+        const int n = 2 << a.diag[d].n_ctrl;
+        for (int i = threadIdx.x; i < n; i += blockDim.x) tab[a.diag[d].tab_off + i] = gt[a.diag[d].src_off + i];
+    }
+    __syncthreads();                                      // the only block-level barrier: member tables staged
     unsigned char *wbase = smem_raw + low_warp_bytes<R, MH>() * warp;
     V16 *Us = reinterpret_cast<V16 *>(wbase);                                      // [NS][32]
     C2 *As = reinterpret_cast<C2 *>(wbase + (size_t)NS * 32 * 16);                 // [4][kLowRow]: a lane reads row lane & 3
@@ -1459,7 +1471,7 @@ __global__ void __launch_bounds__(NW * 32) k_expand_low(const __grid_constant__ 
             const uint64_t x = x_of(lane);
             const uint64_t gi = x | a.rank_bits;
             if (a.tree_out) {
-                const double w = (double)mine.x * (double)mine.x + (double)mine.y * (double)mine.y;
+                const double w = low_weight(mine.x, mine.y);
                 if constexpr (V == 2) {
                     const double w2 = w + __shfl_xor_sync(0xffffffffu, w, 1);
                     if (!(lane & 1)) a.sub_out[x >> 1] = w2;
@@ -1468,7 +1480,6 @@ __global__ void __launch_bounds__(NW * 32) k_expand_low(const __grid_constant__ 
                 }
                 wacc += w;
             }
-            if constexpr (!EMIT) return;
             R pr = mine.x, pi = mine.y;
             low_diag(a, gi, [&](int d, uint32_t idx) { return tab + a.diag[d].tab_off + 2 * idx; }, pr, pi);
             __syncwarp();                                 // the previous batch's phase B is done with the tables
@@ -1545,6 +1556,79 @@ __global__ void __launch_bounds__(NW * 32) k_expand_low(const __grid_constant__ 
             if (lane == 0) a.tree_out[tile * kWarps + warp] = wacc;
         }
     }
+}
+
+// The checkpoint sums of a virtual last pass (DESIGN.md 3): the result is left unwritten, and level 0 is built from the
+// pass's input (the finer level is not stored: the sampler computes the entries it reads, low_sub_entry), with k_expand_low<.., TB, NW>'s association exactly:
+//   - lane i of warp w in tile T holds the inputs x = T 2^TB + b 32 NW + 2w + (i >> 1) 2 NW + (i & 1), batches b in
+//     order, summed from 0.0; warp_sum (xor 16 .. 1) of the lanes is partial[T NW + w];
+//   - level0[j] = left-to-right sum of the 2^g partials from j 2^g on (g = kChunkBits - TB + log2 NW: k_group_sum).
+// A CTA covers one chunk: coalesced 16-byte loads in address order, the weights parked in shared memory; then one thread
+// per partial replays its warp's lanes and butterfly serially (the butterfly is the pairwise sum of the lanes in
+// bit-reversed order), and one thread folds the partials.  One launch, no partials in memory.  (B200, q34: one, two
+// and four chunks per CTA took 0.083, 0.087 and 0.103 ms.)
+constexpr int kSumsThreads = 256;
+template <typename R, int TB, int NW>
+__global__ void __launch_bounds__(kSumsThreads) k_expand_low_sums(const void *__restrict__ in, double *__restrict__ level0) {
+    constexpr int V = sizeof(R) == 4 ? 2 : 1;
+    using V16 = typename VecIO<R, V>::T;
+    constexpr int kVec = (1 << kChunkBits) / V;                         // 16-byte vectors per chunk
+    static_assert(kVec % kSumsThreads == 0, "a CTA loads one whole chunk");
+    constexpr int kLoads = kVec / kSumsThreads;                         // per thread
+    constexpr int NB = (1 << TB) / (32 * NW);                           // batches per warp of the materialising launch
+    constexpr int G = (1 << kChunkBits) / (32 * NB);                    // partials per chunk
+    static_assert(NB >= 1 && G <= kSumsThreads, "one thread per partial");
+    // weight of chunk-local input d at d + (d >> TB): one double of padding per tile spreads a partial's threads over the
+    // banks
+    __shared__ double s_w[(1 << kChunkBits) + ((1 << kChunkBits) >> TB)];
+    __shared__ double s_part[G];
+    auto at = [](uint32_t d) { return d + (d >> TB); };
+    const uint64_t chunk = blockIdx.x;
+    const V16 *src = reinterpret_cast<const V16 *>(in) + chunk * kVec;
+    V16 v[kLoads];
+#pragma unroll
+    for (int k = 0; k < kLoads; ++k) v[k] = __ldg(src + k * kSumsThreads + threadIdx.x);
+#pragma unroll
+    for (int k = 0; k < kLoads; ++k) {
+        const uint32_t idx = k * kSumsThreads + threadIdx.x;                  // vector index within the chunk
+        if constexpr (V == 2) {
+            s_w[at(2 * idx)] = low_weight(v[k].x, v[k].y);
+            s_w[at(2 * idx + 1)] = low_weight(v[k].z, v[k].w);
+        } else {
+            s_w[at(idx)] = low_weight(v[k].x, v[k].y);
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x < G) {
+        const uint32_t k = threadIdx.x;                                        // partial k = (tile k / NW, warp k % NW)
+        const uint32_t base = (k / NW << TB) + 2 * (k % NW);
+        double st[6];                                                          // pairwise-sum stack
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+            const int i = (j & 1) << 4 | (j & 2) << 2 | (j & 4) | (j & 8) >> 2 | (j & 16) >> 4;   // lane: j bit-reversed
+            double acc = 0.0;
+#pragma unroll
+            for (int b = 0; b < NB; ++b) acc += s_w[at(base + b * 32 * NW + (i >> 1) * 2 * NW + (i & 1))];
+            int l = 0;
+#pragma unroll
+            for (; (j >> l) & 1; ++l) acc = st[l] + acc;
+            st[l] = acc;
+        }
+        s_part[k] = st[5];
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double t = 0.0;
+        for (int j = 0; j < G; ++j) t += s_part[j];
+        level0[chunk] = t;
+    }
+}
+
+// the finer level of a virtual pass's tree, written out for qcm_tree_level (the sampler computes its entries in place)
+template <typename R>
+__global__ void __launch_bounds__(kThreads) k_low_sub_entries(const void *in, uint64_t n, double *out) {
+    const uint64_t p = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p < n) out[p] = low_sub_entry<R>(in, p);
 }
 
 // ----------------------------------------------------------------------------------
@@ -1954,6 +2038,7 @@ struct SampleArgs {
                                     // addresses p; logical index = (p >> rot_m) | ((p & (2^rot_m - 1)) << rot_nin)
     int32_t n_levels;               // tree levels above the amplitudes (>= 1)
     const double *sub;              // optional finer level under level[0]: sums over 2^sub_bits amplitudes
+    const void *sub_in;             // ... or, not stored, computed from the rotated pass's input (low_sub_entry)
     int32_t sub_bits;
     int32_t sub_strided;            // sub holds k_chunk_sums' 32 lane partials per chunk (strided groups, see there)
     uint64_t bsub;                  // batch stride of sub, bytes
@@ -2062,10 +2147,11 @@ __global__ void __launch_bounds__(kThreads) k_sample(const __grid_constant__ Sam
             }
             continue;
         }
-        if (a.sub) {
+        if (a.sub || a.sub_in) {
             const uint32_t nsub = 1u << (cb - a.sub_bits);
-            const double *sp = a.sub + (node << (cb - a.sub_bits));      // (fused checkpoint only: never batched)
-            const uint32_t c = warp_pick([&](uint32_t i) { return sp[i]; }, nsub, u, lane);
+            const uint64_t sfirst = node << (cb - a.sub_bits);           // (fused checkpoint only: never batched)
+            const uint32_t c = warp_pick([&](uint32_t i) { return a.sub ? a.sub[sfirst + i] : low_sub_entry<R>(a.sub_in, sfirst + i); },
+                                         nsub, u, lane);
             afirst += (uint64_t)c << a.sub_bits;
             leaf_cnt = 1u << a.sub_bits;
         }
