@@ -347,9 +347,14 @@ class B200Simulator:
                   table_off=em.table(fusion._diag_table_f64(tab)))
         pr.proj = em.finish()
 
-    def _handle(self, n_phys, precision, batch=1):
+    def _handle(self, n_phys, precision, batch=1, deferred=False):
+        """The state handle for this size; `deferred`: the mode its calls run in (execute_deferred keeps a handle in
+        deferred mode between circuits, so that one circuit's readers overlap the next program; any other use leaves
+        it, which orders that use behind them)."""
         key = (n_phys, precision) if batch == 1 else (n_phys, precision, batch)
         h = self._handles.get(key)
+        if h is not None and hasattr(h, 'set_deferred') and getattr(h, 'deferred', False) != deferred:
+            h.set_deferred(deferred)
         if h is None:
             if self._ring is not None and any(rec is not None and not rec['done'] for rec in self._ring['busy']):
                 # the state of a pending execute_deferred() would be released under its running kernels
@@ -361,6 +366,8 @@ class B200Simulator:
             h = _native.Handle(n_phys, precision, self.device, batch=batch) if batch > 1 else \
                 _native.Handle(n_phys, precision, self.device)
             self._handles[key] = h
+            if deferred and hasattr(h, 'set_deferred'):
+                h.set_deferred(True)
         return h
 
     def close(self):
@@ -836,10 +843,13 @@ class B200Simulator:
         blocking execute() where the pipeline does not apply (release width, no shots, variables off the low qubits)."""
         pl = pr.plan
         precision = precision or self.precision
-        h = self._handle(pl.n_phys, precision)
         n = pr.n_vars
-        if not (shots and not pr.virtual and pr.ps is not None and n is not None and n <= min(30, pl.n_phys) and hasattr(h, 'mark')
+        if not (shots and not pr.virtual and pr.ps is not None and n is not None and n <= min(30, pl.n_phys)
                 and all(pl.layout[q] == q for q in range(n))):
+            out = self.execute(pr, shots, seed, stream, precision)
+            return lambda: out
+        h = self._handle(pl.n_phys, precision, deferred=True)
+        if not hasattr(h, 'mark'):
             out = self.execute(pr, shots, seed, stream, precision)
             return lambda: out
         self._last = h
@@ -861,14 +871,14 @@ class B200Simulator:
                                'more are started')
         kb, pb, mb = ring['bufs'][slot]
         mask, value, _ = pr.ps
-        h.set_deferred(True)
         try:
             h.run_program(pl.ops, pl.tables)
             h.sample(shots, seed, stream, pr.clbit_map if len(pr.clbit_map) else None, out=kb.array)
             h.postselect(mask, value, n, out=(pb.array, mb.array))
             ticket = h.mark()
-        finally:
+        except BaseException:
             h.set_deferred(False)
+            raise
         rec = {'done': False}
         ring['busy'][slot] = rec
 

@@ -27,6 +27,25 @@ struct DevBuf {
     size_t cap = 0;
 };
 
+// page-locked staging of the coefficient tables; `done` is recorded after the copies that read it
+struct HostBuf {
+    void *p = nullptr;
+    size_t cap = 0;
+    cudaEvent_t done = nullptr;
+};
+
+// The buffers a deferred circuit's readers (sampler, post-selection, their copies) use after its program was enqueued.
+// The deferred pipeline of a plain handle keeps two sets and gives consecutive programs alternate ones, so that one
+// circuit's readers run on the reader stream while the next program runs on the handle's stream.
+struct BufSet {
+    DevBuf tab_f64, tab_real;       // the program's tables (the virtual pass's descriptor points into them)
+    DevBuf scratch;                 // input copy of a rotated expansion pass (the virtual pass's retained input)
+    DevBuf tree, totals;            // sum tree and its total(s)
+    DevBuf keys, mine, probs, partial;
+    HostBuf stage;
+    cudaEvent_t readers_done = nullptr;   // recorded on the reader stream after the last reader of this set
+};
+
 }  // namespace
 
 struct qcm_sim_s {
@@ -54,12 +73,22 @@ struct qcm_sim_s {
     std::string err;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     qcm_timing timing{};
-    DevBuf tab_f64, tab_real, init_lo, init_hi, probs, partial, keys, mine, tree, ctab, tilectr, subtree;
-    DevBuf scratch;                 // input copy of a rotated expansion pass
-    DevBuf lowpart;                 // its per-CTA partial sums when a CTA covers fewer inputs than a tree chunk
+    BufSet set;                     // the current buffer set
+    BufSet spare;                   // the deferred pipeline's other one (empty outside it)
+    DevBuf &tab_f64 = set.tab_f64, &tab_real = set.tab_real, &scratch = set.scratch, &tree = set.tree, &totals = set.totals,
+           &keys = set.keys, &mine = set.mine, &probs = set.probs, &partial = set.partial;
+    DevBuf init_lo, init_hi, ctab, tilectr, subtree;
+    DevBuf lowpart;                 // per-CTA partial sums of a rotated pass whose CTA covers fewer inputs than a tree chunk
     DevBuf relp1;                   // released-qubit probability tables (qcm_sample_released)
-    DevBuf streams, totals;         // batched sampling: per-point Philox streams and total masses
+    DevBuf streams;                 // batched sampling: per-point Philox streams
     DevBuf errflag;                 // in-place fused exchange: spin-timeout flag
+    // deferred pipeline (plain handle): the readers of a circuit run on `rstream` (non-blocking), after `ev_fork` of the
+    // handle's stream; every call that does not belong to the pipeline first joins them back (`ev_join`, join_readers)
+    cudaStream_t rstream = nullptr;
+    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+    bool readers_pending = false;   // rstream holds work the handle's stream has not waited for
+    bool fork_due = true;           // the handle's stream may hold work rstream has not waited for
+    bool single_set = false;        // the second buffer set could not be allocated: no pipeline
     // rotated storage (QCM_FLAG_ROTATED_OUTPUT_OK): logical index i of the 2^n_active state lives at
     // physical address ((i & (2^rot_nin - 1)) << rot_m) | (i >> rot_nin); rot_m == 0: identity
     int rot_m = 0, rot_nin = 0;
@@ -707,14 +736,14 @@ int launch_block_plan(qcm_handle h, BlockPlan &bp) {
         const size_t smem = bp.tree_smem;
         if (h->prec == QCM_C64) {
             if (V == 2) {
-                if (smem > 48 * 1024) QCM_CUDA(h, cudaFuncSetAttribute(k_expand_tree<float, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                if (smem > 48 * 1024 && (rc = raise_smem_limit(h, (const void *)k_expand_tree<float, 2>))) return rc;
                 k_expand_tree<float, 2><<<bgrid(h, grid), threads, smem, h->stream>>>(bp.trargs);
             } else {
-                if (smem > 48 * 1024) QCM_CUDA(h, cudaFuncSetAttribute(k_expand_tree<float, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                if (smem > 48 * 1024 && (rc = raise_smem_limit(h, (const void *)k_expand_tree<float, 1>))) return rc;
                 k_expand_tree<float, 1><<<bgrid(h, grid), threads, smem, h->stream>>>(bp.trargs);
             }
         } else {
-            if (smem > 48 * 1024) QCM_CUDA(h, cudaFuncSetAttribute(k_expand_tree<double, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            if (smem > 48 * 1024 && (rc = raise_smem_limit(h, (const void *)k_expand_tree<double, 1>))) return rc;
             k_expand_tree<double, 1><<<bgrid(h, grid), threads, smem, h->stream>>>(bp.trargs);
         }
         QCM_CUDA(h, cudaGetLastError());
@@ -1037,15 +1066,28 @@ int upload_tables(qcm_handle h, const double *tables, size_t n_per_point) {
     const size_t n_tables = n_per_point * (size_t)h->batch;      // batched handle: `batch` consecutive table sets
     if (!n_tables) return QCM_OK;
     int rc;
-    if ((rc = ensure(h, h->tab_f64, n_tables * sizeof(double)))) return rc;
-    QCM_CUDA(h, cudaMemcpyAsync(h->tab_f64.p, tables, n_tables * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    if (h->prec == QCM_C64) {
-        std::vector<float> f(n_tables);
+    const size_t b64 = n_tables * sizeof(double), b32 = h->prec == QCM_C64 ? n_tables * sizeof(float) : 0;
+    if ((rc = ensure(h, h->tab_f64, b64))) return rc;
+    if (b32 && (rc = ensure(h, h->tab_real, b32))) return rc;
+    // both uploads go out of the set's page-locked staging buffer, once its previous uploads have been read
+    HostBuf &s = h->set.stage;
+    if (!s.done) QCM_CUDA(h, cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
+    QCM_CUDA(h, cudaEventSynchronize(s.done));
+    if (s.cap < b64 + b32) {
+        if (s.p) QCM_CUDA(h, cudaFreeHost(s.p));
+        s.p = nullptr;
+        s.cap = 0;
+        QCM_CUDA(h, cudaHostAlloc(&s.p, b64 + b32, cudaHostAllocDefault));
+        s.cap = b64 + b32;
+    }
+    memcpy(s.p, tables, b64);
+    QCM_CUDA(h, cudaMemcpyAsync(h->tab_f64.p, s.p, b64, cudaMemcpyHostToDevice, h->stream));
+    if (b32) {
+        float *f = (float *)((char *)s.p + b64);
         for (size_t i = 0; i < n_tables; ++i) f[i] = (float)tables[i];
-        if ((rc = ensure(h, h->tab_real, n_tables * sizeof(float)))) return rc;
-        // pageable source: the runtime stages it before the call returns, so `f` may go out of scope (no synchronisation)
-        QCM_CUDA(h, cudaMemcpyAsync(h->tab_real.p, f.data(), n_tables * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+        QCM_CUDA(h, cudaMemcpyAsync(h->tab_real.p, f, b32, cudaMemcpyHostToDevice, h->stream));
     }                                  // complex128: the fp64 upload IS the table in the state's real type (tabreal)
+    QCM_CUDA(h, cudaEventRecord(s.done, h->stream));
     return QCM_OK;
 }
 
@@ -1253,8 +1295,102 @@ static int launch_gather_inplace(qcm_handle h, const GatherArgs &a, const Gather
     return QCM_OK;
 }
 
-int check_device(qcm_handle h) {
-    QCM_CUDA(h, cudaSetDevice(h->device));
+// The handle's stream waits for everything enqueued on the reader stream so far.
+int join_readers(qcm_handle h) {
+    if (!h->readers_pending) return QCM_OK;
+    QCM_CUDA(h, cudaEventRecord(h->ev_join, h->rstream));
+    QCM_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join, 0));
+    h->readers_pending = false;
+    return QCM_OK;
+}
+
+// Entry of every call.  `join`: the call is not one of the deferred pipeline's, so it runs on the handle's stream behind
+// the readers of earlier circuits (nothing to do inside a reader scope, where an entry point calls another).
+int check_device(qcm_handle h, bool join = true) {
+    int cur = -1;
+    if (cudaGetDevice(&cur) != cudaSuccess || cur != h->device) QCM_CUDA(h, cudaSetDevice(h->device));
+    if (!join || (h->rstream && h->stream == h->rstream)) return QCM_OK;
+    h->fork_due = true;
+    return join_readers(h);
+}
+
+// the deferred pipeline applies: plain handle, second buffer set available
+bool pipelined(const qcm_sim_s *h) { return h->deferred && h->batch == 1 && h->n_global == 0 && !h->single_set; }
+
+// Moves the handle's launches to the reader stream for the scope's lifetime, behind all work of the handle's stream.
+struct ReaderScope {
+    qcm_handle h = nullptr;
+    cudaStream_t main = nullptr;
+    int enter(qcm_handle hd) {
+        h = hd;
+        if (h->fork_due) {
+            QCM_CUDA(h, cudaEventRecord(h->ev_fork, h->stream));
+            QCM_CUDA(h, cudaStreamWaitEvent(h->rstream, h->ev_fork, 0));
+            h->fork_due = false;
+        }
+        main = h->stream;
+        h->stream = h->rstream;
+        h->readers_pending = true;
+        return QCM_OK;
+    }
+    ~ReaderScope() {
+        if (h) h->stream = main;
+    }
+};
+
+void free_set(BufSet &s) {
+    DevBuf *bufs[] = {&s.tab_f64, &s.tab_real, &s.scratch, &s.tree, &s.totals, &s.keys, &s.mine, &s.probs, &s.partial};
+    for (DevBuf *b : bufs) {
+        if (b->p) cudaFree(b->p);
+        *b = DevBuf{};
+    }
+    if (s.stage.p) cudaFreeHost(s.stage.p);
+    if (s.stage.done) cudaEventDestroy(s.stage.done);
+    if (s.readers_done) cudaEventDestroy(s.readers_done);
+    s = BufSet{};
+}
+
+// Start of a pipelined program: hand it the other buffer set, once that set's last readers (two circuits back) are done.
+// The other set is grown to the current one's sizes here, before any launch of the program.  Where that (or the reader
+// stream) cannot be had, the handle keeps one set and the serial order for good.
+int switch_sets(qcm_handle h, bool readers_read_state) {
+    bool ok = true;
+    if (!h->rstream) {
+        ok = cudaStreamCreateWithFlags(&h->rstream, cudaStreamNonBlocking) == cudaSuccess &&
+             cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming) == cudaSuccess &&
+             cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming) == cudaSuccess;
+    }
+    for (BufSet *s : {&h->set, &h->spare})
+        if (ok && !s->readers_done) ok = cudaEventCreateWithFlags(&s->readers_done, cudaEventDisableTiming) == cudaSuccess;
+#ifndef QCM_TEST_ALIAS_SETS
+    const std::pair<DevBuf *, DevBuf *> grow[] = {{&h->spare.tab_f64, &h->tab_f64}, {&h->spare.tab_real, &h->tab_real},
+                                                  {&h->spare.scratch, &h->scratch}, {&h->spare.tree, &h->tree},
+                                                  {&h->spare.totals, &h->totals}, {&h->spare.keys, &h->keys},
+                                                  {&h->spare.mine, &h->mine}, {&h->spare.probs, &h->probs},
+                                                  {&h->spare.partial, &h->partial}};
+    for (const auto &g : grow)
+        if (ok && ensure(h, *g.first, g.second->cap) != QCM_OK) ok = false;
+#endif
+    if (!ok) {
+        cudaGetLastError();
+        free_set(h->spare);
+        h->single_set = true;
+        h->err.clear();
+        return join_readers(h);
+    }
+    QCM_CUDA(h, cudaEventRecord(h->set.readers_done, h->rstream));
+#ifndef QCM_TEST_ALIAS_SETS
+    std::swap(h->set, h->spare);
+#else
+    // test build: both sets share their device buffers (the host staging still alternates, so that the enqueue runs
+    // ahead of the device as in the real build)
+    std::swap(h->set.readers_done, h->spare.readers_done);
+    std::swap(h->set.stage, h->spare.stage);
+#endif
+    QCM_CUDA(h, cudaStreamWaitEvent(h->stream, h->set.readers_done, 0));
+    h->probs_n = 0;                                          // a resident block lived in the other set
+    // the previous circuit's readers read the state itself (its last pass was written): the program waits for them
+    if (readers_read_state) return join_readers(h);
     return QCM_OK;
 }
 
@@ -1396,7 +1532,15 @@ int qcm_destroy(qcm_handle h) {
     if (!h) return QCM_OK;
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->stream);
-    DevBuf *bufs[] = {&h->tab_f64, &h->tab_real, &h->init_lo, &h->init_hi, &h->probs, &h->partial, &h->keys, &h->mine, &h->tree, &h->ctab, &h->tilectr, &h->subtree, &h->scratch, &h->lowpart, &h->relp1, &h->streams, &h->totals, &h->errflag};
+    if (h->rstream) {
+        cudaStreamSynchronize(h->rstream);
+        cudaStreamDestroy(h->rstream);
+    }
+    if (h->ev_fork) cudaEventDestroy(h->ev_fork);
+    if (h->ev_join) cudaEventDestroy(h->ev_join);
+    free_set(h->set);
+    free_set(h->spare);
+    DevBuf *bufs[] = {&h->init_lo, &h->init_hi, &h->ctab, &h->tilectr, &h->subtree, &h->lowpart, &h->relp1, &h->streams, &h->errflag};
     for (DevBuf *b : bufs)
         if (b->p) cudaFree(b->p);
     if (h->own_state && h->state) cudaFree(h->state);
@@ -1520,17 +1664,25 @@ int qcm_tree_level(qcm_handle h, int level, const double **dev_ptr_out, uint64_t
 int qcm_set_deferred(qcm_handle h, int deferred) {
     if (!h) return fail(nullptr, QCM_ERR_INVALID, "handle is NULL");
     h->deferred = deferred != 0;
+    if (!h->deferred) return check_device(h);          // leaving the pipeline: later work runs behind its readers
     return QCM_OK;
 }
 
 int qcm_mark(qcm_handle h, uint64_t *ticket_out) {
     if (!h || !ticket_out) return fail(h, QCM_ERR_INVALID, "NULL argument");
-    int rc = check_device(h);
+    int rc = check_device(h, false);
     if (rc) return rc;
     const uint64_t t = h->n_marks;
     cudaEvent_t &e = h->marks[t % qcm_sim_s::kMarks];
     if (!e) QCM_CUDA(h, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    QCM_CUDA(h, cudaEventRecord(e, h->stream));
+    if (h->readers_pending) {
+        // behind both streams: the reader stream after it has waited for the handle's (later tickets cover earlier ones)
+        ReaderScope rs;
+        if ((rc = rs.enter(h))) return rc;
+        QCM_CUDA(h, cudaEventRecord(e, h->stream));
+    } else {
+        QCM_CUDA(h, cudaEventRecord(e, h->stream));
+    }
     h->n_marks = t + 1;
     *ticket_out = t;
     return QCM_OK;
@@ -1539,7 +1691,7 @@ int qcm_mark(qcm_handle h, uint64_t *ticket_out) {
 int qcm_wait(qcm_handle h, uint64_t ticket) {
     if (!h) return fail(nullptr, QCM_ERR_INVALID, "handle is NULL");
     if (ticket >= h->n_marks) return fail(h, QCM_ERR_INVALID, "ticket %llu was never issued", (unsigned long long)ticket);
-    int rc = check_device(h);
+    int rc = check_device(h, false);
     if (rc) return rc;
     // the slot holds this ticket's event or a later one of the same stream: waiting for it is sufficient either way
     QCM_CUDA(h, cudaEventSynchronize(h->marks[ticket % qcm_sim_s::kMarks]));
@@ -1597,19 +1749,23 @@ int qcm_get_active(qcm_handle h, int *n_active_out) {
 int qcm_run_program(qcm_handle h, const qcm_op *ops, int n_ops, const double *tables, size_t n_tables) {
     if (!h) return fail(nullptr, QCM_ERR_INVALID, "handle is NULL");
     if (n_ops < 0 || (n_ops && !ops) || (n_tables && !tables)) return fail(h, QCM_ERR_INVALID, "NULL program");
-    int rc = check_device(h);
+    const bool pipe = pipelined(h);
+    int rc = check_device(h, !pipe);
     if (rc) return rc;
     h->tree_valid = false;
     h->product_n = -1;
+    const bool prev_virt = h->virt;
     if (h->virt) {
         // the unwritten result depends on this handle's tables and scratch buffer, which this program may reuse: a new
         // state drops it, anything else (which is refused below) writes it out first
         if (n_ops > 0 && ops[0].kind == QCM_OP_INIT_PRODUCT) h->virt = false;
         else if ((rc = materialise_last(h))) return rc;
     }
+    if (pipe && (rc = switch_sets(h, !prev_virt))) return rc;
+    h->fork_due = true;
     bool keep_tree = false;
     h->timing.bytes_read = h->timing.bytes_written = 0;
-    QCM_CUDA(h, cudaEventRecord(h->ev0, h->stream));
+    if (!h->deferred) QCM_CUDA(h, cudaEventRecord(h->ev0, h->stream));
     if ((rc = upload_tables(h, tables, n_tables))) return rc;
     h->op_kind.clear(); h->op_rd.clear(); h->op_wr.clear(); h->op_ms.clear(); h->op_kernel.clear(); h->cur_kernel.clear();
     size_t n_ev = 0;
@@ -1778,10 +1934,10 @@ int qcm_run_program(qcm_handle h, const qcm_op *ops, int n_ops, const double *ta
     }
     h->timing.bytes_read *= (uint64_t)h->batch;
     h->timing.bytes_written *= (uint64_t)h->batch;
-    QCM_CUDA(h, cudaEventRecord(h->ev1, h->stream));
     h->op_ms.assign(h->op_kind.size(), 0.f);
     h->op_ms_pending = h->deferred;
     if (h->deferred) return QCM_OK;          // enqueued; qcm_get_op_profile collects the per-op timings on demand
+    QCM_CUDA(h, cudaEventRecord(h->ev1, h->stream));
     QCM_CUDA(h, cudaEventSynchronize(h->ev1));
     float ms = 0.f;
     QCM_CUDA(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
@@ -1919,7 +2075,7 @@ int qcm_get_op_profile(qcm_handle h, int cap, int32_t *kind_out, float *ms_out, 
     *n_out = n;
     if (h->op_ms_pending && cap > 0 && (size_t)n < h->op_ev.size()) {
         // the last program was only enqueued (deferred mode): wait for its last op and read the events now
-        int rc = check_device(h);
+        int rc = check_device(h, false);
         if (rc) return rc;
         QCM_CUDA(h, cudaEventSynchronize(h->op_ev[n]));
         for (int k = 0; k < n; ++k) QCM_CUDA(h, cudaEventElapsedTime(&h->op_ms[k], h->op_ev[k], h->op_ev[k + 1]));
@@ -1943,40 +2099,45 @@ static int postselect_impl(qcm_handle h, uint64_t mask, uint64_t value, int n_ou
     if (n_out_bits < 0 || n_out_bits > h->n_local || n_out_bits > 30) return fail(h, QCM_ERR_INVALID, "n_out_bits %d out of range", n_out_bits);
     if (value & ~mask) return fail(h, QCM_ERR_INVALID, "value has bits outside mask");
     if (dev && h->batch != 1) return fail(h, QCM_ERR_UNSUPPORTED, "device-resident post-selection on a batched handle: use qcm_postselect_resident");
-    int rc = check_device(h);
-    if (rc) return rc;
-    QCM_CUDA(h, cudaEventRecord(h->ev0, h->stream));
     const uint64_t nprob = 1ull << n_out_bits;
     const uint64_t B = (uint64_t)h->batch;
     const uint64_t local_all = (h->n_local >= 64) ? ~0ull : ((1ull << h->n_local) - 1ull);
     const uint64_t act_all = (1ull << h->n_active) - 1ull;
     const uint64_t rb = rank_bits(h);
     const bool want_probs = probs_out != nullptr || resident;
+    // global (rank) bits and never-materialised bits decide emptiness up front
+    bool empty = ((rb & mask & ~local_all) != (value & ~local_all));
+    if (value & local_all & ~act_all) empty = true;       // demands a 1 on a qubit known |0>
+    const uint64_t lmask = mask & act_all, lval = value & act_all;
+    const int nb = std::min(n_out_bits, h->n_active);
+    const uint64_t out_all = (1ull << nb) - 1ull;
+    const bool contiguous = (lval == 0) && (lmask == (act_all & ~out_all));
+    // rotated storage: logical i lives at ((i & low) << rot_m) | (i >> rot_nin); the kept prefix
+    // (i < 2^nb <= 2^rot_nin) is then the stride-2^rot_m sequence i << rot_m
+    const int pshift = (h->rot_m && nb <= h->rot_nin) ? h->rot_m : 0;
+    const bool prefix = !empty && contiguous && (!h->rot_m || pshift);
+    // deferred pipeline: the prefix post-selection into host buffers is one of the circuit's readers
+    const bool reader = mode == 0 && prefix && pipelined(h) && h->rstream;
+    int rc = check_device(h, !reader);
+    if (rc) return rc;
+    ReaderScope rs;
+    if (reader && (rc = rs.enter(h))) return rc;
+    if (!h->deferred) QCM_CUDA(h, cudaEventRecord(h->ev0, h->stream));
     if (dev) {
         QCM_CUDA(h, cudaMemsetAsync(kept_out, 0, sizeof(double), h->stream));
     } else {
         for (uint64_t y = 0; y < B; ++y) kept_out[y] = 0.0;
-        if (probs_out) memset(probs_out, 0, nprob * B * sizeof(double));
+        if (probs_out && empty) memset(probs_out, 0, nprob * B * sizeof(double));   // else the copy below writes it all
     }
     if (!dev && want_probs) h->probs_n = 0;  // the handle's block buffer is about to be overwritten
-    // global (rank) bits and never-materialised bits decide emptiness up front
-    bool empty = ((rb & mask & ~local_all) != (value & ~local_all));
-    if (value & local_all & ~act_all) empty = true;       // demands a 1 on a qubit known |0>
     if (!dev && want_probs && (rc = ensure(h, h->probs, nprob * B * sizeof(double)))) return rc;
     double *dprobs = want_probs ? (dev ? probs_out : (double *)h->probs.p) : nullptr;
     if (!empty) {
-        const uint64_t lmask = mask & act_all, lval = value & act_all;
-        const int nb = std::min(n_out_bits, h->n_active);
-        const uint64_t out_all = (1ull << nb) - 1ull;
-        const bool contiguous = (lval == 0) && (lmask == (act_all & ~out_all));
-        // rotated storage: logical i lives at ((i & low) << rot_m) | (i >> rot_nin); the kept prefix
-        // (i < 2^nb <= 2^rot_nin) is then the stride-2^rot_m sequence i << rot_m
-        const int pshift = (h->rot_m && nb <= h->rot_nin) ? h->rot_m : 0;
         // a batched sweep spreads its points over the grid: fewer blocks per point
         const int blocks = B > 1 ? std::max(8, (int)((uint64_t)h->num_sms * 8 / B)) : h->num_sms * 4;
         const uint64_t bpart = (uint64_t)(blocks + 1) * sizeof(double), bprobs = nprob * sizeof(double);
         if ((rc = ensure(h, h->partial, bpart * B))) return rc;
-        if (contiguous && (!h->rot_m || pshift)) {
+        if (prefix) {
             const uint64_t count = 1ull << nb;
             if (dprobs && count < nprob) QCM_CUDA(h, cudaMemsetAsync(dprobs, 0, nprob * B * sizeof(double), h->stream));
             double *const part = (double *)h->partial.p;
@@ -2013,8 +2174,8 @@ static int postselect_impl(qcm_handle h, uint64_t mask, uint64_t value, int n_ou
     }
     if (dev) return QCM_OK;                 // results stay on the device, in stream order: no synchronisation
     if (resident) h->probs_n = nprob;
-    QCM_CUDA(h, cudaEventRecord(h->ev1, h->stream));
     if (h->deferred) return QCM_OK;         // kept_out / probs_out (pinned host memory) are valid after qcm_synchronize
+    QCM_CUDA(h, cudaEventRecord(h->ev1, h->stream));
     QCM_CUDA(h, cudaEventSynchronize(h->ev1));
     float ms = 0.f;
     QCM_CUDA(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
@@ -2074,7 +2235,7 @@ static int sample_sharded_impl(qcm_handle h, uint64_t shots, uint64_t seed, uint
     if (rc) return rc;
     if (product_state(h) && n_ranks == 1 && !dev_masses) {
         if (shots == 0) return QCM_OK;
-        QCM_CUDA(h, cudaEventRecord(h->ev0, h->stream));
+        if (!h->deferred) QCM_CUDA(h, cudaEventRecord(h->ev0, h->stream));
         const uint64_t Bp = (uint64_t)h->batch;
         ProductSampleArgs pa{};
         pa.qv = (const double *)h->tab_f64.p + h->product_off;
@@ -2107,8 +2268,8 @@ static int sample_sharded_impl(qcm_handle h, uint64_t shots, uint64_t seed, uint
         if (dev) return QCM_OK;
         QCM_CUDA(h, cudaMemcpyAsync(keys_out, h->keys.p, shots * Bp * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->stream));
         if (mine_out) memset(mine_out, 1, shots);
-        QCM_CUDA(h, cudaEventRecord(h->ev1, h->stream));
         if (h->deferred) return QCM_OK;
+        QCM_CUDA(h, cudaEventRecord(h->ev1, h->stream));
         QCM_CUDA(h, cudaEventSynchronize(h->ev1));
         float pms = 0.f;
         QCM_CUDA(h, cudaEventElapsedTime(&pms, h->ev0, h->ev1));
@@ -2118,7 +2279,7 @@ static int sample_sharded_impl(qcm_handle h, uint64_t shots, uint64_t seed, uint
     if (!h->tree_valid || h->tree_for_active != h->n_active)
         if ((rc = build_tree(h))) return rc;
     if (shots == 0) return QCM_OK;
-    QCM_CUDA(h, cudaEventRecord(h->ev0, h->stream));
+    if (!h->deferred) QCM_CUDA(h, cudaEventRecord(h->ev0, h->stream));
     SampleArgs a{};
     a.state = h->state;
     a.n_active = h->tree_base_bits;
@@ -2198,8 +2359,8 @@ static int sample_sharded_impl(qcm_handle h, uint64_t shots, uint64_t seed, uint
     if (dev) return QCM_OK;                 // keys / mine stay on the device, in stream order
     QCM_CUDA(h, cudaMemcpyAsync(keys_out, h->keys.p, shots * B * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->stream));
     if (mine_out) QCM_CUDA(h, cudaMemcpyAsync(mine_out, h->mine.p, shots, cudaMemcpyDeviceToHost, h->stream));
-    QCM_CUDA(h, cudaEventRecord(h->ev1, h->stream));
     if (h->deferred) return QCM_OK;
+    QCM_CUDA(h, cudaEventRecord(h->ev1, h->stream));
     QCM_CUDA(h, cudaEventSynchronize(h->ev1));
     float ms = 0.f;
     QCM_CUDA(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
@@ -2245,8 +2406,15 @@ int qcm_sample(qcm_handle h, uint64_t shots, uint64_t seed, uint64_t stream_id, 
                uint64_t *keys_out) {
     if (!h) return fail(nullptr, QCM_ERR_INVALID, "handle is NULL");
     if (h->n_global != 0) return fail(h, QCM_ERR_INVALID, "sharded state: use qcm_sample_prepare + qcm_sample_sharded");
+    // deferred pipeline: the sampler on the program's checkpoint tree is one of the circuit's readers (a tree that has
+    // to be built first reads the state: that call stays on the handle's stream)
+    ReaderScope rs;
+    int rc;
+    if (pipelined(h) && h->rstream && !product_state(h) && h->tree_valid && h->tree_for_active == h->n_active) {
+        if ((rc = check_device(h, false)) || (rc = rs.enter(h))) return rc;
+    }
     double mass = 0.0;
-    int rc = qcm_sample_prepare(h, &mass);
+    rc = qcm_sample_prepare(h, &mass);
     if (rc) return rc;
     if (h->deferred && h->batch == 1 && !product_state(h)) {
         // deferred mode: the tree's total was not read back; it is summed on the device (same index order as the host
@@ -2339,8 +2507,8 @@ static int sample_released_impl(qcm_handle h, uint64_t shots, uint64_t seed, uin
     QCM_CUDA(h, cudaGetLastError());
     h->timing.kernel_launches++;
     QCM_CUDA(h, cudaMemcpyAsync(keys_out, h->keys.p, shots * B * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->stream));
-    QCM_CUDA(h, cudaEventRecord(h->ev1, h->stream));
     if (h->deferred) return QCM_OK;
+    QCM_CUDA(h, cudaEventRecord(h->ev1, h->stream));
     QCM_CUDA(h, cudaEventSynchronize(h->ev1));
     float ms = 0.f;
     QCM_CUDA(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));

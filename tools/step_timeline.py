@@ -10,6 +10,13 @@ Writes DIR/step_timeline.pt.trace.json (the raw trace) and DIR/step_timeline.jso
     waiting for the device (wait) and the host's own work (result copies);
   - the card's name and power limit.
 Run it alone: tracing slows the host, so its step period is not the benchmark's.
+
+    python tools/step_timeline.py --out DIR --no-profiler [--steps 200] [--warmup 5]
+
+runs the same loop without the profiler and writes DIR/step_host.json: per step, the host clock around the enqueue
+(execute_deferred) and around the collect (the previous circuit's callable), their medians, the host time per engine
+call, and the loop's wall time per step.  When enqueue + collect minus the wait is close to the wall time per step, the
+host is the limit; otherwise the device is.
 """
 import argparse
 import collections
@@ -39,6 +46,7 @@ def main():
     ap.add_argument('--out', required=True)
     ap.add_argument('--steps', type=int, default=30)
     ap.add_argument('--warmup', type=int, default=5)
+    ap.add_argument('--no-profiler', action='store_true', help='host clocks only (see the module docstring)')
     args = ap.parse_args()
     os.makedirs(args.out, exist_ok=True)
     import torch
@@ -68,6 +76,9 @@ def main():
         sim.execute_deferred(prep, SHOTS, seed=1984, stream=0)()
     torch.cuda.synchronize()
     host.clear()
+    if args.no_profiler:
+        host_only(args, sim, prep, host, torch)
+        return
     enq = col = 0.0
     with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
         pending = None
@@ -134,6 +145,48 @@ def main():
         json.dump(out, f, indent=1)
     print(json.dumps({k: out[k] for k in ('card', 'step_period_ms_median', 'device_busy_ms_median',
                                           'device_idle_ms_median', 'host_work_per_step_ms', 'bound')}))
+
+
+def host_only(args, sim, prep, host, torch):
+    """The pipelined loop of bench.py's device-timed arm with host clocks around each step's enqueue and collect."""
+    enq, col = [], []
+    t_start = time.perf_counter()
+    pending = None
+    for _ in range(args.steps):
+        t0 = time.perf_counter()
+        fin = sim.execute_deferred(prep, SHOTS, seed=1984, stream=0)
+        t1 = time.perf_counter()
+        if pending is not None:
+            pending()
+        col.append(time.perf_counter() - t1)
+        enq.append(t1 - t0)
+        pending = fin
+    t1 = time.perf_counter()
+    pending()
+    col[-1] += time.perf_counter() - t1
+    torch.cuda.synchronize()
+    wall = (time.perf_counter() - t_start) * 1e3 / args.steps
+    sim.op_profile()                                          # what bench.py reads after its loop
+    sim.close()
+    n = args.steps
+    wait = host.get('wait', 0.0) * 1e3 / n
+    ms = lambda v: round(float(v) * 1e3, 4)                   # noqa: E731
+    out = {
+        'card': _card(),
+        'workload': 'q34, complex64, 10^4 shots, execute_deferred back to back (profiler off, host clocks)',
+        'steps': n,
+        'wall_ms_per_step': round(wall, 4),
+        'enqueue_ms_median': ms(np.median(enq)),
+        'collect_ms_median': ms(np.median(col)),
+        'enqueue_ms_mean': ms(np.mean(enq)),
+        'collect_ms_mean': ms(np.mean(col)),
+        'host_ms_per_call': {k: round(v * 1e3 / n, 4) for k, v in sorted(host.items())},
+        'host_work_per_step_ms': round((sum(enq) + sum(col)) * 1e3 / n - wait, 4),
+    }
+    out['bound'] = 'host' if out['host_work_per_step_ms'] >= 0.9 * wall else 'gpu'
+    with open(os.path.join(args.out, 'step_host.json'), 'w') as f:
+        json.dump(out, f, indent=1)
+    print(json.dumps(out))
 
 
 if __name__ == '__main__':
