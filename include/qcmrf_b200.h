@@ -324,6 +324,38 @@ int qcm_run_noisy_small(int device, int precision, int n_circuits, const int32_t
                         const uint64_t *stream_ids, uint64_t shots, uint64_t seed,
                         uint64_t *keys_out, double *device_ms_out);
 
+/* A 1-qubit channel in canonical Kraus form: rho -> sum_i K_i rho K_i^dagger on `qubit`, sum_i K_i^dagger K_i = I
+ * within 1e-10.                                                                                                 */
+typedef struct {
+    double k[4][8];             /* K_i, 2x2 row-major re/im, fp64; entries past n_ops are ignored */
+    int32_t n_ops;              /* 1..4 */
+    int32_t qubit;
+} qcm_kraus;
+
+/* The error after one gate: stages applied in order, each a Pauli channel or a Kraus channel. */
+typedef struct {
+    int32_t n_stages;           /* 1..4 */
+    int32_t kind[4];            /* 0: Pauli channel (index into channels), 1: Kraus (index into krauses) */
+    int32_t index[4];
+    int32_t pad;
+} qcm_gate_error;
+
+/* As qcm_run_noisy_small, but qcm_gate.channel indexes `errors` (-1: no error), and a gate's error applies its
+ * stages in order.  Every stage draws one uniform from Philox4x32-10 keyed (seed ^ Kraus key, stream) at counter
+ * (shot * G_c + g) * 4 + j for stage j of gate g.  A Pauli stage picks its Pauli from the cumulative table; a
+ * Kraus stage picks K_i with probability tr(K_i^dagger K_i rho_q) / sum, rho_q the trajectory's reduced state of
+ * the stage's qubit (never an operator of probability 0), and applies K_i / sqrt(p_i).  A Kraus qubit must be one
+ * of its gate's qubits (target or control).  QCM_ERR_INVALID on a malformed stage, channel or Kraus record (all
+ * checked before any device query) or when a trajectory's norm is not finite and positive.  No CPU fallback. */
+int qcm_run_noisy_small_kraus(int device, int precision, int n_circuits, const int32_t *n_qubits,
+                              const int64_t *gate_begin, const qcm_gate *gates,
+                              const qcm_gate_error *errors, int n_errors,
+                              const qcm_channel *channels, int n_channels,
+                              const qcm_kraus *krauses, int n_kraus,
+                              const int32_t *clbit_qubit, const int32_t *n_clbits, const double *readout,
+                              const uint64_t *stream_ids, uint64_t shots, uint64_t seed,
+                              uint64_t *keys_out, double *device_ms_out);
+
 /* -- batched sweeps ----------------------------------------------------------------- */
 /* A theta / beta sweep over ONE graph (QCMRF's `beta`, /root/reference/QCMRF.py:21,154; BASELINE config 3) is B circuits
  * with the same program structure and different coefficient tables.  A batched handle holds the B states of

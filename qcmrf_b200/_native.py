@@ -44,12 +44,16 @@ SYMBOLS = ['qcm_abi_version', 'qcm_device_count', 'qcm_last_error', 'qcm_create'
            'qcm_postselect_resident', 'qcm_fetch_probs', 'qcm_sample_batched', 'qcm_sample_released_batched',
            'qcm_sample_sharded_devmass', 'qcm_mrf_exact', 'qcm_mrf_last_error', 'qcm_gather_flag_words',
            'qcm_run_gather_block_inplace', 'qcm_set_deferred', 'qcm_host_alloc', 'qcm_host_free',
-           'qcm_tree_total_device', 'qcm_mark', 'qcm_wait', 'qcm_run_batch_small_readout', 'qcm_run_noisy_small', 'qcm_tree_level']
+           'qcm_tree_total_device', 'qcm_mark', 'qcm_wait', 'qcm_run_batch_small_readout', 'qcm_run_noisy_small', 'qcm_tree_level',
+           'qcm_run_noisy_small_kraus']
 
 #: qcm_gate and qcm_channel of include/qcmrf_b200.h (the noisy-shot launch)
 GATE_DTYPE = np.dtype([('m', '<f8', (8,)), ('target', '<i4'), ('ctrl_mask', '<u4'), ('ctrl_value', '<u4'),
                        ('channel', '<i4')])
 CHANNEL_DTYPE = np.dtype([('cum', '<f8', (16,)), ('n_paulis', '<i4'), ('qubit', '<i4', (2,)), ('pad', '<i4')])
+#: qcm_gate_error and qcm_kraus (qcm_run_noisy_small_kraus)
+GATE_ERROR_DTYPE = np.dtype([('n_stages', '<i4'), ('kind', '<i4', (4,)), ('index', '<i4', (4,)), ('pad', '<i4')])
+KRAUS_DTYPE = np.dtype([('k', '<f8', (4, 8)), ('n_ops', '<i4'), ('qubit', '<i4')])
 
 
 def lib():
@@ -83,6 +87,8 @@ def lib():
     L.qcm_run_batch_small_readout.argtypes = [i32, i32, i32, vp, vp, vp, vp, ctypes.c_size_t, vp, vp, vp, vp, vp, vp, vp,
                                               u64, u64, vp, vp, vp, ctypes.POINTER(dbl)]
     L.qcm_run_noisy_small.argtypes = [i32, i32, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, u64, u64, vp, ctypes.POINTER(dbl)]
+    L.qcm_run_noisy_small_kraus.argtypes = [i32, i32, i32, vp, vp, vp, vp, i32, vp, i32, vp, i32, vp, vp, vp, vp, u64,
+                                            u64, vp, ctypes.POINTER(dbl)]
     L.qcm_state_ptr.argtypes = [vp, ctypes.POINTER(vp), ctypes.POINTER(u64)]
     L.qcm_tree_level.argtypes = [vp, i32, ctypes.POINTER(vp), ctypes.POINTER(u64), ctypes.POINTER(i32)]
     L.qcm_set_active.argtypes = [vp, i32]
@@ -475,23 +481,34 @@ def run_batch_small(plans, clbit_maps, ps, shots, seed, precision='double', devi
     return keys, plist, kept, ms.value
 
 
-def run_noisy_small(encoded, shots, seed, precision='double', device=0, stream_ids=None):
-    """Noisy shots of noise.EncodedNoise programs (qcm_run_noisy_small): one trajectory per shot.  Returns
-    (keys[n][shots] uint64, device_ms)."""
+def _noisy_records(encoded, kraus):
+    """Flat qcm_gate, qcm_channel (and for `kraus`, qcm_gate_error and qcm_kraus) arrays of noise.EncodedNoise
+    programs, record indices made global; with the per-circuit clbit maps and readout tables."""
     n = len(encoded)
     nq = np.array([e.n_qubits for e in encoded], dtype=np.int32)
     gate_begin = np.concatenate([[0], np.cumsum([e.n_gates for e in encoded])]).astype(np.int64)
     gates = np.zeros(int(gate_begin[-1]), dtype=GATE_DTYPE)
-    chans, coff = [], 0
+    chans, errs, krs = [], [], []
+    coff = eoff = koff = 0
     for i, e in enumerate(encoded):
         g = gates[gate_begin[i]:gate_begin[i + 1]]
         g['m'], g['target'], g['ctrl_mask'], g['ctrl_value'] = e.matrix, e.target, e.ctrl_mask, e.ctrl_value
-        g['channel'] = np.where(e.channel >= 0, e.channel + coff, -1)
+        g['channel'] = np.where(e.channel >= 0, e.channel + (eoff if kraus else coff), -1)
         ch = np.zeros(len(e.n_paulis), dtype=CHANNEL_DTYPE)
         ch['cum'], ch['n_paulis'], ch['qubit'] = e.cum, e.n_paulis, e.chan_qubits
         chans.append(ch)
+        if kraus:
+            er = np.zeros(len(e.err_n_stages), dtype=GATE_ERROR_DTYPE)
+            er['n_stages'], er['kind'] = e.err_n_stages, e.err_kind
+            er['index'] = e.err_index + np.where(e.err_kind == 1, koff, coff)
+            kr = np.zeros(len(e.kraus_n_ops), dtype=KRAUS_DTYPE)
+            kr['k'], kr['n_ops'], kr['qubit'] = e.kraus_ops, e.kraus_n_ops, e.kraus_qubit
+            errs.append(er)
+            krs.append(kr)
+            eoff += len(er)
+            koff += len(kr)
         coff += len(ch)
-    channels = np.concatenate(chans) if chans else np.zeros(0, dtype=CHANNEL_DTYPE)
+    cat = lambda parts, dt: np.concatenate(parts) if parts else np.zeros(0, dtype=dt)
     cq = np.full((n, 64), -1, dtype=np.int32)
     ncl = np.zeros(n, dtype=np.int32)
     ro = np.zeros((n, 64, 2))
@@ -499,15 +516,42 @@ def run_noisy_small(encoded, shots, seed, precision='double', device=0, stream_i
         cq[i, :e.n_clbits] = e.clbit_map
         ncl[i] = e.n_clbits
         ro[i] = e.readout
-    keys = np.empty((n, int(shots)), dtype=np.uint64)
+    return (nq, gate_begin, gates, cat(chans, CHANNEL_DTYPE), cat(errs, GATE_ERROR_DTYPE), cat(krs, KRAUS_DTYPE),
+            cq, ncl, ro)
+
+
+def run_noisy_small(encoded, shots, seed, precision='double', device=0, stream_ids=None):
+    """Noisy shots of noise.EncodedNoise programs whose errors are single Pauli channels (qcm_run_noisy_small): one
+    trajectory per shot.  Returns (keys[n][shots] uint64, device_ms)."""
+    nq, gate_begin, gates, channels, _, _, cq, ncl, ro = _noisy_records(encoded, False)
+    keys = np.empty((len(encoded), int(shots)), dtype=np.uint64)
     sid = None if stream_ids is None else np.ascontiguousarray(stream_ids, dtype=np.uint64)
     ms = ctypes.c_double()
     prec = QCM_C64 if precision in ('single', 'c64', 32) else QCM_C128
-    rc = lib().qcm_run_noisy_small(int(device), prec, n, _ptr(nq), _ptr(gate_begin), _ptr(gates), _ptr(channels),
-                                   len(channels), _ptr(cq), _ptr(ncl), _ptr(ro) if ro.any() else None, _ptr(sid),
-                                   int(shots), int(seed), _ptr(keys), ctypes.byref(ms))
+    rc = lib().qcm_run_noisy_small(int(device), prec, len(encoded), _ptr(nq), _ptr(gate_begin), _ptr(gates),
+                                   _ptr(channels), len(channels), _ptr(cq), _ptr(ncl), _ptr(ro) if ro.any() else None,
+                                   _ptr(sid), int(shots), int(seed), _ptr(keys), ctypes.byref(ms))
     if rc:
         raise NativeError(rc, 'qcm_run_noisy_small failed')
+    return keys, ms.value
+
+
+def run_noisy_small_kraus(encoded, shots, seed, precision='double', device=0, stream_ids=None):
+    """Noisy shots of noise.EncodedNoise programs through their error records (qcm_run_noisy_small_kraus): errors
+    of up to 4 stages, Pauli or 1-qubit Kraus.  Any encoding runs here (a Pauli-only one as one-stage records).
+    Returns (keys[n][shots] uint64, device_ms)."""
+    nq, gate_begin, gates, channels, errors, krauses, cq, ncl, ro = _noisy_records(encoded, True)
+    keys = np.empty((len(encoded), int(shots)), dtype=np.uint64)
+    sid = None if stream_ids is None else np.ascontiguousarray(stream_ids, dtype=np.uint64)
+    ms = ctypes.c_double()
+    prec = QCM_C64 if precision in ('single', 'c64', 32) else QCM_C128
+    rc = lib().qcm_run_noisy_small_kraus(int(device), prec, len(encoded), _ptr(nq), _ptr(gate_begin), _ptr(gates),
+                                         _ptr(errors), len(errors),
+                                         _ptr(channels), len(channels), _ptr(krauses), len(krauses), _ptr(cq),
+                                         _ptr(ncl), _ptr(ro) if ro.any() else None, _ptr(sid), int(shots), int(seed),
+                                         _ptr(keys), ctypes.byref(ms))
+    if rc:
+        raise NativeError(rc, 'qcm_run_noisy_small_kraus failed')
     return keys, ms.value
 
 

@@ -541,7 +541,8 @@ class B200Simulator:
         to any circuit, which then runs exactly as without a model.  A circuit is noisy when an error with a
         non-identity probability above 0 follows one of its gates or reads one of its measured qubits.  A noisy call
         runs every circuit on the small-circuit path (no sweeps, no release width; ValueError above small_max
-        qubits): circuits with gate errors as one trajectory per shot (qcm_run_noisy_small), the others through the
+        qubits): circuits with gate errors as one trajectory per shot -- through qcm_run_noisy_small when every error
+        that applies is one Pauli channel, through qcm_run_noisy_small_kraus otherwise -- the others through the
         ideal batched kernel, their keys flipped by their readout errors on the device.  Noisy experiments have
         counts and no exact pmf or success probability."""
         progs = [ir.lower(c) for c in circs]
@@ -554,16 +555,19 @@ class B200Simulator:
         if big:
             raise ValueError('noisy shots need circuits of at most %d qubits (circuit %d has %d)'
                              % (small_max, big[0], progs[big[0]].n_qubits))
-        traj = [i for i, e in enumerate(enc) if e.gate_noisy]
-        if traj:
-            keys, ms = _native.run_noisy_small([enc[i] for i in traj], shots, seed, precision=precision,
-                                               device=self.device, stream_ids=[sid(i) for i in traj])
+        for kraus, run, path in ((False, _native.run_noisy_small, 'noisy_trajectories'),
+                                 (True, _native.run_noisy_small_kraus, 'noisy_trajectories_kraus')):
+            traj = [i for i, e in enumerate(enc) if e.gate_noisy and e.kraus == kraus]
+            if not traj:
+                continue
+            keys, ms = run([enc[i] for i in traj], shots, seed, precision=precision, device=self.device,
+                           stream_ids=[sid(i) for i in traj])
             for j, i in enumerate(traj):
                 p = progs[i]
                 entries[i] = {'circuit': circs[i], 'name': p.name,
                               'counts': _keys_to_counts(keys[j], p.n_clbits) if shots else None, 'probs': None,
                               'kept': None,
-                              'meta': {'path': 'noisy_trajectories', 'noise': True, 'n_qubits': p.n_qubits,
+                              'meta': {'path': path, 'noise': True, 'n_qubits': p.n_qubits,
                                        'gates': enc[i].n_gates, 'channels': len(enc[i].n_paulis),
                                        'noisy_device_ms': ms, 'philox_stream': sid(i)}}
         rest = [i for i, e in enumerate(enc) if not e.gate_noisy]
